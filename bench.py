@@ -5,6 +5,7 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
       --master-port P bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...     # the CPU restatement of the reference's path
+  python bench.py ... --dump-outputs DIR   # also write the last timed step's results as .npy
 
 One "step" = one pass of the hot path (backbone + ConvDet + interpret_output +
 filter_prediction/NMS) over one batch of synthetic 1242x375 images.  Headline line: SqueezeDet,
@@ -56,7 +57,15 @@ def parse_args():
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--no-other-configs', action='store_true',
                   help='skip BASELINE configs 3-5 and the strong-scaling leg')
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write what the last timed step of the headline run computed (rank 0) '
+                       'as DIR/<name>.npy, float32/float64, at most 64 MB in all')
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl == 'reference':
+    ap.error('--dump-outputs writes what the GPU path computed; --impl reference has no such output')
+  return args
 
 
 def measured_peaks():
@@ -357,14 +366,49 @@ class Runner:
     self.barrier()
     return self.max_over_ranks(dt * 1e3) / steps
 
-  def measure(self, steps, warmup, global_images, want_f32_feed=False):
+  def fetch_outputs(self, budget=64 << 20):
+    """The results of the last forward, as a caller of the device-resident path reads them:
+    det_boxes [B,A,4], det_probs [B,A], det_class [B,A] (float32) and the filtered records
+    [B,max_dets,7] (anchor, cls, prob, cx, cy, w, h; float64) with their counts [B].  Over
+    `budget` bytes, the det_* arrays keep a fixed seeded sample of anchors, listed in
+    anchor_sample.npy."""
+    self.stream.synchronize()
+    r = self.model.results_device()
+    B, A, md = self.B, int(self.model.det_probs.shape[1]), r['max_dets']
+
+    def fetch(ptr, dtype, shape):
+      out = np.empty(shape, dtype)
+      self._lib.check(self.lib.sqdet_memcpy_d2h(out.ctypes.data, ptr, out.nbytes, None))
+      self._lib.check(self.lib.sqdet_stream_sync(self.local, None))
+      return out
+    dets = fetch(r['dets'], self._lib.DET_DTYPE, (B, md))
+    arrays = {
+        'det_boxes': fetch(r['det_boxes'], np.float32, (B, A, 4)),
+        'det_probs': fetch(r['det_probs'], np.float32, (B, A)),
+        'det_class': fetch(r['det_class'], np.int64, (B, A)).astype(np.float32),
+        'records': np.stack([dets[f].astype(np.float64) for f in dets.dtype.names], axis=-1),
+        'counts': fetch(r['counts'], np.int32, (B,)).astype(np.float64)}
+    det_bytes = B * A * 6 * 4
+    rest = arrays['records'].nbytes + arrays['counts'].nbytes
+    if det_bytes + rest > budget:
+      k = max(1, (budget - rest - 8 * A) // (B * 6 * 4))
+      keep = np.sort(np.random.default_rng(0).choice(A, size=min(k, A), replace=False))
+      for name in ('det_boxes', 'det_probs', 'det_class'):
+        arrays[name] = np.ascontiguousarray(arrays[name][:, keep])
+      arrays['anchor_sample'] = keep.astype(np.float64)
+    return arrays
+
+  def measure(self, steps, warmup, global_images, want_f32_feed=False, fetch=False):
     """-> dict(value, ms_per_step, e2e...).  `global_images` = images the whole job processes
-    per step (world * B for weak scaling, the real global batch for strong scaling)."""
+    per step (world * B for weak scaling, the real global batch for strong scaling).  fetch=True
+    adds 'outputs': fetch_outputs() of the last timed step (rank 0)."""
     _lib = self._lib
     for _ in range(max(warmup, 3)):
       self.step_device()
     ms = self.timed_device(steps) / steps
     out = {'ms_per_step': ms, 'value': global_images / (ms * 1e-3)}
+    if fetch and self.rank == 0:
+      out['outputs'] = self.fetch_outputs()       # before the e2e steps overwrite the results
     ms_e2e = self.timed_e2e(_lib.IMG_U8, self.pinned_u8.ptr, steps)
     out['e2e'] = {'value': global_images / (ms_e2e * 1e-3), 'unit': 'images/sec',
                   'h2d_bytes_per_step': int(self.pinned_u8.array.nbytes),
@@ -495,7 +539,7 @@ def run_ours(args):
   sampler = ClockSampler(local)
   if rank == 0:
     sampler.start()
-  res = main.measure(args.steps, W, world * B, want_f32_feed=True)
+  res = main.measure(args.steps, W, world * B, want_f32_feed=True, fetch=bool(args.dump_outputs))
   gather_ok = main.check_gather() if world > 1 else None
   if world > 1:
     main.model.set_gather_in_forward(False)     # what follows is rank-local (no collective)
@@ -506,6 +550,10 @@ def run_ours(args):
       main.step_device()
       stream.synchronize()
   clocks = sampler.stop() if rank == 0 else None
+  if 'outputs' in res:
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, a in res.pop('outputs').items():
+      np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
 
   roofline = per_op = None
   if rank == 0:
@@ -551,14 +599,13 @@ def run_ours(args):
       plans = [('squeezeDet+', 20, world * 20, 'weak'),
                ('squeezeDet+', max(shard.shard_sizes(20, world)), 20, 'strong'),
                ('vgg16', max(shard.shard_sizes(gb_v, world)), gb_v, 'strong')]
-    steps_o = max(5, min(args.steps, 10))
     for net, b, gimg, mode in plans:
       r = Runner(args, net, b, rank, world, local, stream, new_ident())
-      m = r.measure(steps_o, 3, gimg)
+      m = r.measure(args.steps, 3, gimg)
       row = {'net': net, 'workload': workload_name(net, args.width, args.height, b),
              'n_gpus': world, 'scaling': mode, 'global_batch': gimg, 'batch_per_gpu': b,
              'value': m['value'], 'unit': 'images/sec', 'ms_per_step': m['ms_per_step'],
-             'steps': steps_o, 'e2e': m['e2e']}
+             'steps': args.steps, 'e2e': m['e2e']}
       if world > 1:
         r.model.set_gather_in_forward(False)
       if rank == 0:

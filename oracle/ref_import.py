@@ -7,8 +7,8 @@ What imports and runs as-is under Python 3.12 once ``tensorflow`` and
   * ``utils.util.nms / batch_iou / iou``                 (src/utils/util.py:9-76)
   * ``nn_skeleton.ModelSkeleton.filter_prediction``      (src/nn_skeleton.py:696-734)
   * ``config.kitti_*_config()`` incl. ``set_anchors``    (src/config/*.py)
-Used by ``tests/golden/make_golden.py`` (fixture generator) and by
-``tests/test_oracle_pinning.py`` (live check, skipped when the tree is absent).
+Used by ``tests/golden/make_golden.py``, which records the reference's outputs as the fixtures
+under ``tests/golden/`` that ``tests/test_oracle_pinning.py`` checks the oracle against.
 """
 from __future__ import annotations
 

@@ -460,6 +460,10 @@ static int prepare_params(sqdet_engine* e) {
       if (rc) return rc;
     }
   }
+  // cudaMemcpy from pageable host memory may return before its DMA has landed, and the forward
+  // runs on non-blocking streams that do not wait for the legacy stream: every upload above (and
+  // the plan-time ones of sqdet_finalize) must be complete before a kernel reads it
+  SQ_CUDA(cudaStreamSynchronize(nullptr));
   e->params_dirty = false;
   // weights changed -> any captured graph still points at the same buffers, so it stays valid
   return SQDET_OK;
@@ -1314,6 +1318,7 @@ int sqdet_set_box_scale(sqdet_engine* e, const float* xy_scales) {
     SQ_CUDA(cudaDeviceSynchronize());
     SQ_CUDA(cudaMemcpy(e->d_scales, xy_scales, sizeof(float) * n, cudaMemcpyHostToDevice));
     SQ_CUDA(cudaMemcpy(e->d_scales + n, xy_scales, sizeof(float) * n, cudaMemcpyHostToDevice));
+    SQ_CUDA(cudaStreamSynchronize(nullptr));   // landed before the next forward's stream reads it
   }
   if (on != e->rescale_on) {
     e->rescale_on = on;

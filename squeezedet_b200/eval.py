@@ -10,7 +10,7 @@ filtered (filter_prediction + NMS on original-image coordinates, eval.py:86-87) 
 `sqdet_submit_frames(..., order=eval, rescale=1)` call; corner format + score go into
 all_boxes[cls][image].  Then the KITTI detection files are written
 (src/dataset/kitti.py:100-127) and the reference's unmodified `evaluate_object` binary
-(built by tools/build_kitti_eval.sh) is invoked and its stats_*_ap.txt parsed
+(built by oracle/build_kitti_eval.sh) is invoked and its stats_*_ap.txt parsed
 (kitti.py:129-159).  The TensorBoard summaries and the checkpoint-polling loop
 (eval.py:171-239) are not rebuilt.
 """
@@ -77,8 +77,9 @@ def detections_to_all_boxes(records, count, scale, num_classes):
   return out
 
 
-EVAL_TOOL = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'dataset', 'kitti-eval',
-                         'cpp', 'evaluate_object')   # built by tools/build_kitti_eval.sh
+# the reference's scorer as __graft_entry__.build() / oracle/build_kitti_eval.sh compile it
+EVAL_TOOL = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle',
+                         '_ref', 'evaluate_object')
 
 
 def eval_once(flags):
@@ -136,7 +137,7 @@ def eval_once(flags):
       print('    {}: {:.3f}'.format(name, ap))
     print('    Mean average precision: {:.3f}'.format(float(np.mean(aps))))
   else:
-    print('KITTI scorer binary not found ({}; build it with tools/build_kitti_eval.sh); '
+    print('KITTI scorer binary not found ({}; build it with oracle/build_kitti_eval.sh); '
           'detection files are in {}'.format(tool, det_dir))
   return all_boxes, aps, names
 

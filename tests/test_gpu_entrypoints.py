@@ -131,7 +131,8 @@ def test_eval_once_reference_order_files_and_scorer(tmp_path, gpu_device):
         k += 1
   # the reference's unmodified scorer ran and its AP files were parsed (kitti.py:129-159)
   if not os.path.exists(sq_eval.EVAL_TOOL):
-    pytest.skip('scorer binary absent: __graft_entry__.build() compiles it where /root/reference exists')
+    pytest.skip('scorer binary absent: __graft_entry__.build() compiles it into oracle/_ref where '
+                'the reference checkout exists')
   assert aps is not None and len(aps) == 3 * mc.CLASSES and names[0] == 'car_easy'
   # evaluate_object writes stats_<class>_ap.txt for exactly the classes that occur in the detection
   # files (its eval_car / eval_pedestrian / eval_cyclist flags, evaluate_object.cpp:695-776)

@@ -1,14 +1,13 @@
-"""The oracle's numpy half against (a) the committed fixtures produced by the
-reference's own functions (tests/golden/make_golden.py) and (b) the live reference
-import when /root/reference is present (dev container only)."""
+"""The oracle's numpy half against the committed fixtures produced by the reference's own
+functions (tests/golden/make_golden.py)."""
 import hashlib
+import os
 
 import numpy as np
-import pytest
 
 import oracle
 from oracle import postproc as P
-from oracle import ref_import
+from golden.make_golden import filter_trials, trial_sha256
 
 
 def _run_oracle(c):
@@ -70,24 +69,20 @@ def test_set_anchors_matches_reference_fixtures(anchors_golden):
     assert a[0].tolist() == g['first'] and a[-1].tolist() == g['last']
 
 
-@pytest.mark.skipif(not ref_import.available(), reason='reference tree not mounted')
-def test_live_reference_import_agrees():
-  ns = ref_import.load()
-  rng = np.random.default_rng(7)
-  for trial in range(60):
-    n = int(rng.integers(1, 400))
-    boxes = np.stack([rng.uniform(0, 1242, n), rng.uniform(0, 375, n),
-                      rng.uniform(5, 300, n), rng.uniform(5, 200, n)], 1).astype(np.float32)
-    probs = rng.permutation(np.linspace(0.001, 0.999, n)).astype(np.float32)
-    cls = rng.integers(0, 3, n).astype(np.int64)
-    top_n = int(rng.choice([64, 0, 1000, 10]))
-    fb, fp, fc = ref_import.ref_filter_prediction(ns, boxes, probs, cls, 3, top_n, 0.005, 0.4)
+def test_reference_filter_prediction_recorded_outputs():
+  """60 seeded cases through the oracle, against what the reference's own filter_prediction
+  returned for them (reference_filter.npz: the input rows it kept, in its output order)."""
+  z = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'reference_filter.npz'))
+  ends = np.cumsum(z['counts'])
+  trials = list(filter_trials())
+  assert len(trials) == len(ends) == 60
+  for t, (boxes, probs, cls, top_n) in enumerate(trials):
+    assert trial_sha256(boxes, probs, cls, top_n) == z['input_sha256'][t], t
+    rows = z['rows'][ends[t] - z['counts'][t]:ends[t]].astype(np.int64)
     ob, op, oc, _ = oracle.filter_prediction(boxes, probs, cls, 3, top_n, 0.005, 0.4)
-    assert fc == oc
-    assert all(np.array_equal(x, y) for x, y in zip(fb, ob))
-    assert [float(x) for x in fp] == [float(x) for x in op]
-  for fn, (w, h, gh, gw, shapes) in CONFIGS.items():
-    assert np.array_equal(ns.configs[fn]().ANCHOR_BOX, oracle.set_anchors(w, h, gh, gw, shapes))
+    assert oc == cls[rows].tolist(), t
+    assert len(ob) == len(rows) and all(np.array_equal(x, boxes[r]) for x, r in zip(ob, rows)), t
+    assert [float(x) for x in op] == [float(x) for x in probs[rows]], t
 
 
 def test_interpret_output_hand_case():
