@@ -222,15 +222,6 @@ int sqdet_conv2d(const float* x_dev, const float* w_hwio_dev, const float* bias_
                  int B, int H, int W, int Cin, int Cout, int size, int stride,
                  int padding, int relu, int y_cstride, int y_coff, int math_mode,
                  void* stream);
-/* The halo-tile tensor-core path of a 3x3, stride-1, SAME convolution (csrc/halo_tc.cu; the
- * plan the engine picks for the ConvDet head, src/nets/squeezeDet.py:73-78) as a stage-isolated
- * call: same arguments as sqdet_conv2d without size/stride/padding/math_mode.  Returns
- * SQDET_ERR_UNSUPPORTED for shapes that kernel does not take (Cin % 16, channel-window rules).
- * Synchronises the stream (test / debug entry).                                          */
-int sqdet_conv3x3_halo(const float* x_dev, const float* w_hwio_dev, const float* bias_dev,
-                       const float* scale_dev, const float* shift_dev, float* y_dev, int B,
-                       int H, int W, int Cin, int Cout, int relu, int y_cstride, int y_coff,
-                       void* stream);
 /* SqueezeDet._fire_layer (src/nets/squeezeDet.py:81-106; same in squeezeDetPlus.py) as ONE
  * call: y[..., :E1] = relu(1x1_e1(q)+b), y[..., E1:] = relu(3x3_e3(q)+b), q = relu(1x1_s(x)+b).
  * x [B,H,W,Cin], kernels HWIO, y [B,H,W,E1+E3].  With SQDET_MATH_TF32X3_TC and a shape the

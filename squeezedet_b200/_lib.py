@@ -94,7 +94,6 @@ SIGNATURES = {
     'sqdet_gathered_dev': (_i, [_vp, C.POINTER(_vp), C.POINTER(C.c_int64),
                                 C.POINTER(C.c_int32)]),
     'sqdet_fire': (_i, [_fp] * 8 + [_i] * 8 + [_vp]),
-    'sqdet_conv3x3_halo': (_i, [_fp] * 6 + [_i] * 8 + [_vp]),
     'sqdet_conv2d': (_i, [_fp, _fp, _fp, _fp, _fp, _fp] + [_i] * 12 + [_vp]),
     'sqdet_maxpool_nhwc': (_i, [_fp, _fp] + [_i] * 7 + [_vp]),
     'sqdet_preprocess_u8': (_i, [_vp, _i, _i, _fp, _i, _i, _vp, _i, _vp]),

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
 #include <string>
 #include "../../include/sqdet_b200.h"
 
@@ -25,17 +26,18 @@ int  cuda_fail(cudaError_t err, const char* what);
   } while (0)
 
 
-// ---- programmatic dependent launch (PDL) --------------------------------------------------
-// The forward is a chain of ~20 kernels, each reading what the previous one wrote.  With the
-// programmatic-stream-serialization launch attribute a kernel may be SCHEDULED while its
-// predecessor still runs: its prologue (mbarrier init, tensor-memory allocation, tensor-map
-// fetch) overlaps the predecessor's ragged last wave, and `griddepcontrol.wait` then holds every
-// thread until the predecessor has completed and flushed.  Every kernel of the forward calls
-// pdl_trigger() first (lets ITS successor be scheduled) and pdl_wait() before touching global
-// memory; both are no-ops for a plain launch.  The engine switches the attribute on per thread
-// around sqdet_forward (never for the first kernel, whose input comes from a copy).
-void set_pdl_launch(bool on);
-bool pdl_launch();
+// ---- environment switches (INTEGRATION.md §5) ---------------------------------------------
+// Every SQDET_* variable the library reads goes through these, as the initializer of a
+// function-local `static const`: read once, on first use, thread-safe.
+inline const char* env_str(const char* name) { return getenv(name); }
+inline int env_int(const char* name, int dflt) {
+  const char* a = env_str(name);
+  return a ? atoi(a) : dflt;
+}
+inline float env_float(const char* name, float dflt) {
+  const char* a = env_str(name);
+  return a ? (float)atof(a) : dflt;
+}
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
@@ -45,20 +47,8 @@ inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  if (pdl_launch()) {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-  }
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
-
-#ifdef __CUDACC__
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-#endif
 
 // ---- TF NHWC geometry (SURVEY App. A.1; tf.nn.conv2d / tf.nn.max_pool) ------------------
 struct Geom {

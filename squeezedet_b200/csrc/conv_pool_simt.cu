@@ -56,8 +56,6 @@ struct ConvPoolParams {
 template <int KS, int NT, int MINB>
 __global__ void __launch_bounds__(NT, MINB)
 conv_pool_simt_kernel(const ConvPoolParams p) {
-  pdl_trigger();
-  pdl_wait();
   constexpr int PH = 2 * (CT_H - 1) + KS;          // input patch rows
   constexpr int PW = 2 * (CT_W - 1) + KS;          // input patch cols (pixels)
   constexpr int K = KS * KS * 3;

@@ -24,8 +24,6 @@ conv_simt_kernel(const float* __restrict__ x, const float* __restrict__ w,
                  int B, int H, int W, int Cin, int Cout, int ksz, int stride,
                  int pad_t, int pad_l, int Ho, int Wo, int relu, int y_cstride,
                  int y_coff) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ __align__(16) float As[BK][BM + 4];
   __shared__ __align__(16) float Bs[BK][BN];
 

@@ -8,8 +8,7 @@
 //
 // GEMM view per CTA:  D[128 pixels, N] += A[128 pixels, K] * W[K, N]
 //   M tile  = an 8 x 16 patch of output pixels of one image (TMEM lane = pixel); 128 consecutive
-//             pixels of the flattened B*H*W list when the launch holds only 1x1 convs; the conv
-//             pixels under a block of pooling windows when a stride-2 max-pool is fused
+//             pixels of the flattened B*H*W list when the launch holds only 1x1 convs
 //   N       = one chunk of output channels (multiple of 16, <= 128; TMEM column = channel)
 //   K       = taps x Cin, walked as (tap, 32- or 16-channel chunk)
 //   A       : TMA tiled load of the NHWC activation tensor, box {KC ch, 16 w, 8 h, 1 n} at
@@ -42,9 +41,8 @@
 //   running sums (up to 128 per thread) must stay out of local memory.
 // Pipelines: full[s] (TMA -> splitter), split[s] (splitter -> MMA), empty[s]
 //   (tcgen05.commit -> TMA), tfull[group][b] (tcgen05.commit -> drain), tempty[b] (drain -> MMA).
-// Opt-in variants kept for measurement (all parity-green, all slower today, DESIGN.md 4.1):
-//   weight-tile TMA multicast over CTA clusters, CTA-pair MMA (cta_group::2), fused max-pool
-//   epilogue; -DSQDET_ABLATE builds can switch pipeline pieces off (tools/ablate.sh).
+// Variants measured and removed (weight multicast over CTA clusters, CTA-pair MMA, a second
+//   splitter warpgroup, a fused max-pool epilogue): DESIGN.md 4.1.
 // Roofline: SqueezeDet fire2-9 are HBM-bound even fused (AI 24-95 FLOP/B fp32 I/O),
 //   fire10/11 ~ridge, ConvDet tensor-bound (SURVEY.md §8d); 3xTF32 costs 3 MMAs at the
 //   TF32 rate per algorithmic MAC.
@@ -62,7 +60,6 @@
 
 #include "common.cuh"
 #include "conv_tc.cuh"
-#include "halo_tc.cuh"
 #include "tc_ptx.cuh"
 
 namespace sqdet {
@@ -72,9 +69,6 @@ constexpr int TILE_H = 8, TILE_W = 16, TILE_M = TILE_H * TILE_W;   // 128 pixels
 constexpr int NUM_THREADS = 512;       // 4 warpgroups: {TMA, MMA, 2 spare} | splitter | drain A | drain B
 constexpr int MAX_CHUNKS = 16;
 constexpr int MAX_N = 128;          // output channels per item (register-resident running sums)
-constexpr int POOL_MAX_N = 64;      // ... when a max-pool is fused (conv tile staged per drain group)
-constexpr int POOL_MAX_GROUPS = POOL_MAX_N / 32;
-constexpr int POOL_STAGE_BYTES = POOL_MAX_GROUPS * (16384 + 4096);   // conv + pooled tiles
 constexpr int MAX_STAGES = 8;
 constexpr int GATHER_PITCH = 128;   // floats between patch rows in the stage (gather mode)
 
@@ -95,7 +89,6 @@ struct TcChunk {
 struct TcParams {
   CUtensorMap tmA;
   CUtensorMap tmW;
-  CUtensorMap tmWs;     // weight slice map for cluster multicast: box {KC, 2N/cluster} rows
   CUtensorMap tmY;      // output tensor, box {32 ch, 16 w, 8 h, 1}, SWIZZLE_128B (TMA-store epilogue)
   const float* bias;    // may be null
   const float* scale;   // may be null (frozen BN)
@@ -109,9 +102,8 @@ struct TcParams {
   float bias_comp;      // first-order compensation of the accumulator's truncation bias, per chained MMA
   int ntiles;           // B * tiles_h * tiles_w
   int tma_store;        // 1: epilogue stages 32-channel groups in smem and issues TMA stores
-  // conv tile (rows of the M=128 MMA tile): ct_h x ct_w output pixels (8x16, or 7x17 / 8x16
-  // when a 3x3 / 2x2 stride-2 max-pool is fused into the epilogue); tile step in conv pixels
-  int ct_h, ct_w, step_h, step_w, org_h, org_w;   // origin = tile*step - org
+  // conv tile (rows of the M=128 MMA tile): ct_h x ct_w output pixels, tile t starts at t * ct
+  int ct_h, ct_w;
   int sq_w, sq_h;       // TMA-store epilogue: offset of drain warp q's 32-pixel slab in the tile
   // gather mode (first layer: 3x3 conv over a 3-channel image): the A tile is the im2col
   // of an input patch; the producer fetches the patch row by row with 1-D TMA loads (rows of a
@@ -121,18 +113,10 @@ struct TcParams {
   int gather;           // 1 = gather mode
   int g_H, g_W, g_stride, g_pad_t, g_pad_l;
   int g_ph, g_box;      // patch rows; floats fetched per patch row (patch columns * 3, padded to 4)
-  // fused max-pool (0 = none, else window 2 or 3; stride 2): pooled tile pt_h x pt_w, pooled dims
-  int pool, pt_h, pt_w, Hp, Wp;
   int store_ring;       // per-warp TMA-store staging tiles (2, or 1 to buy one more pipeline stage)
-  int ablate;           // profiling builds only (-DSQDET_ABLATE): bitmask of pipeline pieces to skip
-  int two_cta;          // 1: CTA-pair MMA (cta_group::2), implies cluster == 2
-  int cluster;          // CTAs per cluster (1, 2 or 4): weight tiles are TMA-multicast across it
-  int exp_mode;         // timing experiments only (SQDET_TC_EXP): 1 no fence, 2 no store, 4 no STS
-  int two_split;        // 1: warpgroup 3 is a SECOND operand splitter (alternate stages) and warpgroup 2 the
-                        // only drain group: thin-N, K-heavy launches whose stage the splitter paced
   // static schedule (launches whose chunks differ in cost): sched[0 .. nbins] = first entry of each
-  // cluster's item list, followed by the lists (longest-processing-time-first assignment);
-  // null = round-robin `item = cluster id + k * clusters`
+  // CTA's item list, followed by the lists (longest-processing-time-first assignment);
+  // null = round-robin `item = CTA id + k * CTAs`
   const int* sched;
   long long* dbg;       // optional per-CTA cycle counters (SQDET_TC_DEBUG=1), else null
   int y_cstride, relu;
@@ -154,40 +138,15 @@ struct TcParams {
     }                                                       \
   } while (0)
 
-// One pooled 16-byte channel chunk: max over the PK x PK window (stride 2) of conv-tile rows.
-// Conv staging: per 32-channel group a 128-row x 128 B tile (16 KB, 128B-swizzled), conv tile
-// width 14 + PK; pooled staging: per group a (pt_h*8)-row x 128 B tile (4 KB apart).
-template <int PK>
-__device__ __forceinline__ void pool_unit(uint32_t conv_base, uint32_t pool_base, int u, int n_pp) {
-  constexpr int CTW = 14 + PK;
-  const int k2 = u & 7;
-  const int pu = u >> 3;
-  const int jg = pu / n_pp, pp = pu - jg * n_pp;
-  const int py = pp >> 3, px = pp & 7;
-  const uint32_t tc = conv_base + (uint32_t)(jg * 16384);
-  float4 m = make_float4(-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F);
-#pragma unroll
-  for (int a = 0; a < PK; ++a)
-#pragma unroll
-    for (int b = 0; b < PK; ++b) {
-      const int rr = (2 * py + a) * CTW + 2 * px + b;
-      const float4 q4 = lds128(tc + (uint32_t)(rr * 128 + ((k2 ^ (rr & 7)) << 4)));
-      m.x = fmaxf(m.x, q4.x); m.y = fmaxf(m.y, q4.y);
-      m.z = fmaxf(m.z, q4.z); m.w = fmaxf(m.w, q4.w);
-    }
-  sts128(pool_base + (uint32_t)(jg * 4096 + pp * 128 + ((k2 ^ (pp & 7)) << 4)), m);
-}
-
 // ---------------------------------------------------------------------------------------------
-template <int KC, bool TWO, bool GATHER>
+template <int KC, bool GATHER>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ TcParams p) {
   extern __shared__ uint8_t smem_dyn[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) &
                                              ~uintptr_t(1023));
   constexpr int A_BYTES = TILE_M * KC * 4;
-  // B tile bytes held by THIS CTA: all N rows, or N/2 in CTA-pair mode
-  const int B_BYTES = (TWO ? p.N / 2 : p.N) * KC * 4;
+  const int B_BYTES = p.N * KC * 4;
   const int STAGE_BYTES = A_BYTES + 2 * B_BYTES;   // [A raw][B hi][B lo]
   const int S = p.stages;
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)S * STAGE_BYTES);
@@ -210,52 +169,36 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
   const uint32_t par_b = smem_b + (uint32_t)(reinterpret_cast<uint8_t*>(s_par) - smem);
   const uint32_t out_b = smem_b + (uint32_t)(s_out - smem);
 
-  pdl_trigger();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // Work decomposition: a cluster of C CTAs walks "super-items" = C consecutive tiles of one
-  // chunk in lockstep, so that every weight tile is fetched from L2 once per cluster and
-  // multicast into all C shared memories.  Tiles past the end are clamped (recomputed, not stored).
-  const int C = p.cluster;
-  const uint32_t crank = C > 1 ? cluster_ctarank() : 0u;
-  const int cid = (int)blockIdx.x / C, n_clusters = (int)gridDim.x / C;
-  const int spc = (p.ntiles + C - 1) / C;              // super-items per chunk
-  const int total_items = spc * p.nchunks;             // super-items
-  const uint16_t cmask = (uint16_t)((1u << C) - 1u);
+  // Work decomposition: items are (chunk, tile) pairs, item = chunk * ntiles + tile.
+  const int cta = (int)blockIdx.x, n_ctas = (int)gridDim.x;
+  const int total_items = p.ntiles * p.nchunks;
   const int G = p.seg_stages;
-  // this cluster's items: entries [k_begin, k_end) of the static schedule, or round-robin
-  const int k_begin = p.sched ? __ldg(p.sched + cid) : 0;
-  const int k_end = p.sched ? __ldg(p.sched + cid + 1)
-                            : (total_items - cid + n_clusters - 1) / n_clusters;
+  // this CTA's items: entries [k_begin, k_end) of the static schedule, or round-robin
+  const int k_begin = p.sched ? __ldg(p.sched + cta) : 0;
+  const int k_end = p.sched ? __ldg(p.sched + cta + 1) : (total_items - cta + n_ctas - 1) / n_ctas;
 #define SQ_FOR_ITEMS(...)                                                                \
   for (int k_ = k_begin, nxt_ = (p.sched && k_begin < k_end) ? __ldg(p.sched + k_begin) : 0, \
-           item = p.sched ? nxt_ : cid;                                                  \
+           item = p.sched ? nxt_ : cta;                                                  \
        k_ < k_end;                                                                       \
-       ++k_, item = p.sched ? nxt_ : cid + k_ * n_clusters __VA_ARGS__)                  \
+       ++k_, item = p.sched ? nxt_ : cta + k_ * n_ctas __VA_ARGS__)                      \
     if (p.sched && k_ + 1 < k_end ? (nxt_ = __ldg(p.sched + k_ + 1), true) : true)
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < S; ++s) {
       mbar_init(&full[s], 1);
-      mbar_init(&split[s], TWO ? 256 : 128);  // pair mode: both CTAs' splitters arrive at the leader
-      mbar_init(&empty[s], TWO ? 1u : (uint32_t)C);   // commit arrivals (pair mode: one multicast)
+      mbar_init(&split[s], 128);
+      mbar_init(&empty[s], 1);
     }
     for (int b = 0; b < 4; ++b) mbar_init(&tfull[b], 1);
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(&tempty[b], TWO ? 256 : 128);
-    }
+    for (int b = 0; b < 2; ++b) mbar_init(&tempty[b], 128);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 1) {
-    if (TWO) tmem_alloc_2(tmem_slot, (uint32_t)p.tmem_cols);
-    else tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
   tc_fence_before();
   __syncthreads();
-  if (C > 1) cluster_sync_all();           // peers' barriers exist before anyone multicasts
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // prologue done (overlapped the previous kernel's tail under PDL): from here on global memory
-  pdl_wait();
 
   // Register re-balancing between the warpgroups (launch bound: 168/thread) happens at the top
   // of every role branch, so that ptxas sees one register budget per branch.
@@ -271,12 +214,11 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
       long long w_empty = 0;
       const long long t_begin = clock64();
       SQ_FOR_ITEMS() {
-        const TcChunk ck = p.chunk[item / spc];
-        int tile = (item % spc) * C + (int)crank;
-        if (tile >= p.ntiles) tile = p.ntiles - 1;
+        const TcChunk ck = p.chunk[item / p.ntiles];
+        int tile = item % p.ntiles;
         const int tw = tile % p.tiles_w;
         tile /= p.tiles_w;
-        const int h0 = (tile % p.tiles_h) * p.step_h - p.org_h, w0 = tw * p.step_w - p.org_w;
+        const int h0 = (tile % p.tiles_h) * p.ct_h, w0 = tw * p.ct_w;
         const int img = tile / p.tiles_h;
         const int iters = ck.tap_count * ck.kc_count;
         const uint32_t a_bytes = (uint32_t)(p.ct_h * p.ct_w * KC * 4);   // the TMA box
@@ -286,19 +228,11 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
           if (++st_i == S) { st_i = 0; st_ph ^= 1u; }
           SQ_TIMED_WAIT(w_empty, &empty[s], ph ^ 1u);
           uint8_t* st = smem + (size_t)s * STAGE_BYTES;
-#ifdef SQDET_ABLATE
-          mbar_expect_tx(&full[s], ((p.ablate & 4) ? 0u : a_bytes) +
-                                       ((p.ablate & 2) ? 0u : (uint32_t)(2 * B_BYTES)));
-#else
           mbar_expect_tx(&full[s], (GATHER ? (uint32_t)(p.g_ph * p.g_box * 4) : a_bytes) +
                                        (uint32_t)(2 * B_BYTES));
-#endif
           const int tl = i / ck.kc_count, kc = ck.kc_begin + (i - tl * ck.kc_count);
           const int tap = ck.tap_begin + tl;
           const int dy = tap / ck.ksize, dx = tap - dy * ck.ksize;
-#ifdef SQDET_ABLATE
-          if (!(p.ablate & 4))
-#endif
           if (GATHER) {
             // patch rows at a 512-byte pitch in the stage's A region.  TMA needs a 16-byte aligned global start: every row is fetched from its start
             // rounded down to 4 floats (the splitter adds the 0..3 float offset back); rows
@@ -313,26 +247,8 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
             tma_load_4d(st, &p.tmA, &full[s], kc * KC, w0 + dx - ck.pad, h0 + dy - ck.pad, img);
           }
           const int row = ck.w_row_base + i * p.N;
-#ifdef SQDET_ABLATE
-          if (p.ablate & 2) continue;
-#endif
-          if (TWO) {
-            // this CTA's half (rows crank*N/2 ...) of the hi and of the lo tile
-            const int r0 = (int)crank * (p.N / 2);
-            tma_load_2d(st + A_BYTES, &p.tmWs, &full[s], 0, row + r0);
-            tma_load_2d(st + A_BYTES + B_BYTES, &p.tmWs, &full[s], 0, row + r0 + p.lo_row_offset);
-          } else if (C == 1) {
-            tma_load_2d(st + A_BYTES, &p.tmW, &full[s], 0, row);
-            tma_load_2d(st + A_BYTES + B_BYTES, &p.tmW, &full[s], 0, row + p.lo_row_offset);
-          } else {
-            // this CTA fetches slice `crank` of the stacked [hi (N rows); lo (N rows)] tile and
-            // multicasts it to the whole cluster
-            const int srows = 2 * p.N / C;
-            const int r0 = (int)crank * srows;
-            const int which = r0 / p.N, rr = r0 - which * p.N;
-            tma_load_2d_mc(st + A_BYTES + which * B_BYTES + rr * KC * 4, &p.tmWs, &full[s], 0,
-                           row + rr + which * p.lo_row_offset, cmask);
-          }
+          tma_load_2d(st + A_BYTES, &p.tmW, &full[s], 0, row);
+          tma_load_2d(st + A_BYTES + B_BYTES, &p.tmW, &full[s], 0, row + p.lo_row_offset);
         }
       }
       if (p.dbg) {
@@ -344,97 +260,76 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
    } else if (warp == 1) {
     // ================================ MMA issuer =========================================
     // The whole warp walks the loop (warp-uniform addresses/descriptors live in uniform
-    // registers); only lane 0 issues tcgen05.mma / tcgen05.commit.  In CTA-pair mode only the
-    // leader CTA (cluster rank 0) issues, for both CTAs.
-    if (!TWO || crank == 0) {
-      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(p.N >> 3) << 17) |
-                             ((uint32_t)((TWO ? 2 * TILE_M : TILE_M) >> 4) << 24);
-      const uint32_t smem_base = __shfl_sync(0xffffffffu, smem_u32(smem), 0);
-      const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);   // provably warp-uniform
-      const uint64_t desc_hi = make_desc<KC>(0) & 0xFFFFFFFF00000000ull;   // layout/SBO/version
-      const uint32_t desc_lo0 = (uint32_t)(make_desc<KC>(0) & 0xFFFFFFFFull);  // LBO field
-      int it = 0, g = 0, st_i = 0, n_item = 0;
-      uint32_t st_ph = 0;
-      long long w_split = 0, w_tempty = 0;
-      SQ_FOR_ITEMS(, ++n_item) {
-        const TcChunk ck = p.chunk[item / spc];
-        const int iters = ck.tap_count * ck.kc_count;
-        const int owner = p.two_split ? 0 : (n_item & 1);   // drain group of this item
-        for (int i0 = 0; i0 < iters; i0 += G, ++g) {
-          const int buf = g & 1;
-          SQ_TIMED_WAIT(w_tempty, &tempty[buf], (((uint32_t)g >> 1) & 1u) ^ 1u);   // buffer drained
+    // registers); only lane 0 issues tcgen05.mma / tcgen05.commit.
+    const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(p.N >> 3) << 17) |
+                           ((uint32_t)(TILE_M >> 4) << 24);
+    const uint32_t smem_base = __shfl_sync(0xffffffffu, smem_u32(smem), 0);
+    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);   // provably warp-uniform
+    const uint64_t desc_hi = make_desc<KC>(0) & 0xFFFFFFFF00000000ull;   // layout/SBO/version
+    const uint32_t desc_lo0 = (uint32_t)(make_desc<KC>(0) & 0xFFFFFFFFull);  // LBO field
+    int it = 0, g = 0, st_i = 0, n_item = 0;
+    uint32_t st_ph = 0;
+    long long w_split = 0, w_tempty = 0;
+    SQ_FOR_ITEMS(, ++n_item) {
+      const TcChunk ck = p.chunk[item / p.ntiles];
+      const int iters = ck.tap_count * ck.kc_count;
+      const int owner = n_item & 1;             // drain group of this item
+      for (int i0 = 0; i0 < iters; i0 += G, ++g) {
+        const int buf = g & 1;
+        SQ_TIMED_WAIT(w_tempty, &tempty[buf], (((uint32_t)g >> 1) & 1u) ^ 1u);   // buffer drained
+        tc_fence_after();
+        const uint32_t d_tmem = tmem_u + (uint32_t)(buf * p.N);
+        const int i1 = (i0 + G < iters) ? (i0 + G) : iters;
+        for (int i = i0; i < i1; ++i, ++it) {
+          const int s = st_i;
+          const uint32_t ph = st_ph;
+          if (++st_i == S) { st_i = 0; st_ph ^= 1u; }
+          SQ_TIMED_WAIT(w_split, &split[s], ph);
           tc_fence_after();
-          const uint32_t d_tmem = tmem_u + (uint32_t)(buf * p.N);
-          const int i1 = (i0 + G < iters) ? (i0 + G) : iters;
-          for (int i = i0; i < i1; ++i, ++it) {
-            const int s = st_i;
-            const uint32_t ph = st_ph;
-            if (++st_i == S) { st_i = 0; st_ph ^= 1u; }
-            SQ_TIMED_WAIT(w_split, &split[s], ph);
-            tc_fence_after();
-            // B descriptor low words (start address >> 4 | LBO), +2 per 32-byte K step;
-            // A operand: TMEM slot s = 2*KC columns [hi | lo], 8 columns per K step
-            const uint32_t b_hi =
-                desc_lo0 | ((smem_base + (uint32_t)(s * STAGE_BYTES) + (uint32_t)A_BYTES) >> 4);
-            const uint32_t b_lo = b_hi + (uint32_t)(B_BYTES >> 4);
-            const uint32_t a_hi = tmem_u + (uint32_t)(2 * p.N + s * 2 * KC);
-            const uint32_t a_lo = a_hi + KC;
-            if (elect_one()) {
+          // B descriptor low words (start address >> 4 | LBO), +2 per 32-byte K step;
+          // A operand: TMEM slot s = 2*KC columns [hi | lo], 8 columns per K step
+          const uint32_t b_hi =
+              desc_lo0 | ((smem_base + (uint32_t)(s * STAGE_BYTES) + (uint32_t)A_BYTES) >> 4);
+          const uint32_t b_lo = b_hi + (uint32_t)(B_BYTES >> 4);
+          const uint32_t a_hi = tmem_u + (uint32_t)(2 * p.N + s * 2 * KC);
+          const uint32_t a_lo = a_hi + KC;
+          if (elect_one()) {
 #pragma unroll
-              for (int j = 0; j < KC / 8; ++j) {
-                const uint64_t dbh = desc_hi | (uint64_t)(b_hi + 2 * j);
-                const uint64_t dbl = desc_hi | (uint64_t)(b_lo + 2 * j);
-                if (TWO) {
-                  umma_tf32_ts_2(d_tmem, a_lo + 8 * j, dbh, idesc, (i != i0 || j != 0) ? 1u : 0u);
-                  umma_tf32_ts_2(d_tmem, a_hi + 8 * j, dbl, idesc, 1u);
-                  umma_tf32_ts_2(d_tmem, a_hi + 8 * j, dbh, idesc, 1u);
-                } else {
-                  umma_tf32_ts(d_tmem, a_lo + 8 * j, dbh, idesc, (i != i0 || j != 0) ? 1u : 0u);
-#ifdef SQDET_ABLATE
-                  if (p.ablate & 32) continue;
-#endif
-                  umma_tf32_ts(d_tmem, a_hi + 8 * j, dbl, idesc, 1u);
-                  umma_tf32_ts(d_tmem, a_hi + 8 * j, dbh, idesc, 1u);
-                }
-              }
-              if (TWO) umma_commit_2(&empty[s]);    // frees the stage in both CTAs of the pair
-              else if (C == 1) umma_commit(&empty[s]);   // frees the smem stage once the MMAs read it
-              else umma_commit_mc(&empty[s], cmask);   // ... in every CTA of the cluster
+            for (int j = 0; j < KC / 8; ++j) {
+              const uint64_t dbh = desc_hi | (uint64_t)(b_hi + 2 * j);
+              const uint64_t dbl = desc_hi | (uint64_t)(b_lo + 2 * j);
+              umma_tf32_ts(d_tmem, a_lo + 8 * j, dbh, idesc, (i != i0 || j != 0) ? 1u : 0u);
+              umma_tf32_ts(d_tmem, a_hi + 8 * j, dbl, idesc, 1u);
+              umma_tf32_ts(d_tmem, a_hi + 8 * j, dbh, idesc, 1u);
             }
-            __syncwarp();
-          }
-          if (elect_one()) {                       // segment complete -> its drain group
-            if (TWO) umma_commit_2(&tfull[owner * 2 + buf]);
-            else umma_commit(&tfull[owner * 2 + buf]);
+            umma_commit(&empty[s]);               // frees the smem stage once the MMAs read it
           }
           __syncwarp();
         }
-      }
-      if (p.dbg && lane == 0) {
-        p.dbg[blockIdx.x * 12 + 1] = w_split;
-        p.dbg[blockIdx.x * 12 + 2] = w_tempty;
+        if (elect_one()) umma_commit(&tfull[owner * 2 + buf]);   // segment complete -> its drain group
+        __syncwarp();
       }
     }
+    if (p.dbg && lane == 0) {
+      p.dbg[blockIdx.x * 12 + 1] = w_split;
+      p.dbg[blockIdx.x * 12 + 2] = w_tempty;
+    }
    }   // warps 2-3 of warpgroup 0 are spare: straight to the teardown barrier
-  } else if (warp < 8 || (p.two_split && warp >= 12)) {
+  } else if (warp < 8) {
     // ================================ operand splitter ====================================
-    // (two_split: warpgroups 1 and 3 take alternate stages; BOTH wait on every full[s] in order - an
-    // mbarrier waiter that skips phases can mistake phase n-2 for phase n)
     asm volatile("setmaxnreg.dec.sync.aligned.u32 80;");
-    const int sgroup = warp >= 12 ? 1 : 0;
     const int t = threadIdx.x & 127;   // 0..127
     int it = 0, st_i = 0;
     uint32_t st_ph = 0;
     long long w_full = 0;
     SQ_FOR_ITEMS() {
-      const TcChunk ck = p.chunk[item / spc];
+      const TcChunk ck = p.chunk[item / p.ntiles];
       const int iters = ck.tap_count * ck.kc_count;
       for (int i = 0; i < iters; ++i, ++it) {
         const int s = st_i;
         const uint32_t ph = st_ph;
         if (++st_i == S) { st_i = 0; st_ph ^= 1u; }
         SQ_TIMED_WAIT(w_full, &full[s], ph);
-        if (p.two_split && (it & 1) != sgroup) continue;
         // row t of the raw tile (KC*4 bytes, swizzled 16-byte chunks) -> registers ->
         // a_hi / a_lo -> TMEM slot s, lane t (this warp owns lanes 32*(warp%4)..+31)
         if (KC == 32 && GATHER) {
@@ -442,11 +337,10 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
           // patch rows; taps outside the image (SAME padding), taps 27..31 and rows past the
           // tile are zero
           const uint32_t patch = smem_b + (uint32_t)(s * STAGE_BYTES);
-          int tile = (item % spc) * C + (int)crank;
-          if (tile >= p.ntiles) tile = p.ntiles - 1;
+          int tile = item % p.ntiles;
           const int tw = tile % p.tiles_w;
           tile /= p.tiles_w;
-          const int h0 = (tile % p.tiles_h) * p.step_h - p.org_h, w0 = tw * p.step_w - p.org_w;
+          const int h0 = (tile % p.tiles_h) * p.ct_h, w0 = tw * p.ct_w;
           const int img = tile / p.tiles_h;
           const int r_h = t / p.ct_w, r_w = t - r_h * p.ct_w;
           const bool live = r_h < p.ct_h;
@@ -488,17 +382,13 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
           }
           tmem_wait_st();
           tc_fence_before();
-          if (TWO) mbar_arrive_remote(&split[s], 0u);
-          else mbar_arrive(&split[s]);
+          mbar_arrive(&split[s]);
           continue;
         }
         const uint32_t arow = smem_b + (uint32_t)(s * STAGE_BYTES + t * (KC * 4));
         const int sw = (KC == 32) ? (t & 7) : ((t >> 1) & 3);
         const uint32_t a_slot = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) +
                                 (uint32_t)(2 * p.N + s * 2 * KC);
-#ifdef SQDET_ABLATE
-        if (!(p.ablate & 1))
-#endif
 #pragma unroll
         for (int hblk = 0; hblk < KC / 16; ++hblk) {       // 16 columns at a time
           uint32_t hi[16], lo[16];
@@ -521,39 +411,34 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
         }
         tmem_wait_st();
         tc_fence_before();             // order the TMEM writes before the barrier hand-off
-        if (TWO) mbar_arrive_remote(&split[s], 0u);   // the leader CTA's barrier
-        else mbar_arrive(&split[s]);
+        mbar_arrive(&split[s]);
       }
     }
-    if (p.dbg && t == 0 && sgroup == 0) p.dbg[blockIdx.x * 12 + 3] = w_full;
+    if (p.dbg && t == 0) p.dbg[blockIdx.x * 12 + 3] = w_full;
   } else {
     // ============================ segment drain + epilogue ================================
     asm volatile("setmaxnreg.inc.sync.aligned.u32 192;");
     // two drain groups (warps 8-11 and 12-15) take alternate items
-    const int dgroup = (warp >= 12) ? 1 : 0;     // (two_split: warpgroup 3 never gets here)
-    const int ngroups = p.two_split ? 1 : 2;
+    const int dgroup = (warp >= 12) ? 1 : 0;
     const int q = warp & 3;                      // TMEM lane quarter this warp may access
     const int r = q * 32 + lane;                 // accumulator row = pixel within the tile
     const int tt = threadIdx.x - 256 - 128 * dgroup;   // 0..127 within the drain group
     float acc[MAX_N];
     int g = 0;
-    long long w_tfull = 0, c_epi = 0, c_stw = 0, c_pool = 0, c_par = 0;
+    long long w_tfull = 0, c_epi = 0, c_stw = 0, c_par = 0;
     int n_item = 0, n_own = 0, n_store = 0;
     uint32_t use0 = 0u, use1 = 0u;               // own segments seen per TMEM buffer
     SQ_FOR_ITEMS(, ++n_item) {
-      const TcChunk ck = p.chunk[item / spc];
+      const TcChunk ck = p.chunk[item / p.ntiles];
       const int iters = ck.tap_count * ck.kc_count;
-      if ((n_item % ngroups) != dgroup) {
+      if ((n_item & 1) != dgroup) {
         g += (iters + G - 1) / G;                // segments of an item the other group drains
         continue;
       }
-      int tile = (item % spc) * C + (int)crank;
-      const bool tile_valid = tile < p.ntiles;
-      if (!tile_valid) tile = p.ntiles - 1;
+      int tile = item % p.ntiles;
       const int tw = tile % p.tiles_w;
       tile /= p.tiles_w;
-      const int th_i = tile % p.tiles_h;
-      const int h0 = th_i * p.step_h - p.org_h, w0 = tw * p.step_w - p.org_w;
+      const int h0 = (tile % p.tiles_h) * p.ct_h, w0 = tw * p.ct_w;
       const int img = tile / p.tiles_h;
       const int ncols = (ck.ch_count + 15) & ~15;
       // stage this item's bias / scale / shift in smem (one element per drain thread); the
@@ -582,9 +467,6 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
         // scale the segment sum back while adding it (one FFMA instead of the FADD).
         const int seg_st = (iters - i0) < G ? (iters - i0) : G;
         const float seg_gain = 1.f + p.bias_comp * (float)(3 * (KC / 8) * seg_st);
-#ifdef SQDET_ABLATE
-        if (!(p.ablate & 8))
-#endif
 #pragma unroll
         for (int c0 = 0; c0 < MAX_N; c0 += 16) {
           if (c0 < ncols) {                      // warp-uniform
@@ -597,123 +479,58 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
           }
         }
         tc_fence_before();
-        if (TWO) mbar_arrive_remote(&tempty[buf], 0u);
-        else mbar_arrive(&tempty[buf]);          // buffer may be overwritten by segment g+2
+        mbar_arrive(&tempty[buf]);               // buffer may be overwritten by segment g+2
       }
       // ---- epilogue: bias [, affine], relu, 128-bit stores of this pixel's channel run ----
       const long long t_epi = p.dbg ? clock64() : 0;
       const int r_h = r / p.ct_w, r_w = r - r_h * p.ct_w;
       const int oh = h0 + r_h, ow = w0 + r_w;
-      const bool pix_ok = (r_h < p.ct_h) && oh >= 0 && ow >= 0 && oh < p.Ho && ow < p.Wo;
-#ifdef SQDET_ABLATE
-      if (p.ablate & 16) continue;
-#endif
+      const bool pix_ok = (r_h < p.ct_h) && oh < p.Ho && ow < p.Wo;
       if (p.tma_store) {
         // TMEM-drained sums -> (+bias [*scale+shift], relu) -> swizzled smem tiles -> TMA
         // stores.  The TMA unit writes whole 128-byte lines asynchronously and clips ragged
-        // tiles / the channel tail; the drain warps never wait on global memory.
+        // tiles / the channel tail; the drain warps never wait on global memory.  Each warp
+        // owns tile rows 2q, 2q+1 (its 32 TMEM lanes) and stores them itself: no CTA-level
+        // barrier, only __syncwarp.  Ring of two 4 KB tiles per warp.
         const bool affine = p.scale != nullptr;
         const float lo_clip = p.relu ? 0.f : -CUDART_INF_F;
-        if (!p.pool) {
-          // ---- plain: each warp owns tile rows 2q, 2q+1 (its 32 TMEM lanes) and stores them
-          // itself: no CTA-level barrier, only __syncwarp.  Ring of two 4 KB tiles per warp.
 #pragma unroll
-          for (int jg = 0; jg < MAX_N / 32; ++jg) {
-            if (jg * 32 < ck.ch_count) {                  // warp-uniform
-              if (lane == 0) {
-                const long long t0 = p.dbg ? clock64() : 0;
-                if (p.store_ring == 2) tma_store_wait_read_le1();   // tile used 2 stores ago is free
-                else tma_store_wait_read_all();
-                if (p.dbg) c_stw += clock64() - t0;
-              }
-              __syncwarp();
-              const uint32_t tile_w = out_b + (uint32_t)((dgroup * 4 + q) * (4096 * p.store_ring) +
-                                                         (p.store_ring == 2 ? (n_store & 1) * 4096 : 0));
-#pragma unroll
-              for (int k = 0; k < 8; ++k) {
-                const int c = jg * 32 + k * 4;
-                const float4 b0 = lds128(par + 4u * (uint32_t)c);
-                float o[4] = {acc[c] + b0.x, acc[c + 1] + b0.y, acc[c + 2] + b0.z,
-                              acc[c + 3] + b0.w};
-                if (affine) {
-                  const float4 s0 = lds128(par + 4u * (uint32_t)(MAX_N + c));
-                  const float4 h0v = lds128(par + 4u * (uint32_t)(2 * MAX_N + c));
-                  o[0] = o[0] * s0.x + h0v.x; o[1] = o[1] * s0.y + h0v.y;
-                  o[2] = o[2] * s0.z + h0v.z; o[3] = o[3] * s0.w + h0v.w;
-                }
-                float4 v;
-                v.x = fmaxf(o[0], lo_clip); v.y = fmaxf(o[1], lo_clip);
-                v.z = fmaxf(o[2], lo_clip); v.w = fmaxf(o[3], lo_clip);
-                sts128(tile_w + (uint32_t)(lane * 128 + ((k ^ (lane & 7)) << 4)), v);
-              }
-              fence_async_proxy();
-              __syncwarp();
-              if (lane == 0 && tile_valid)
-                tma_store_4d(tile_w, &p.tmY, ck.y_coff + jg * 32, w0 + q * p.sq_w, h0 + q * p.sq_h, img);
-              ++n_store;
+        for (int jg = 0; jg < MAX_N / 32; ++jg) {
+          if (jg * 32 < ck.ch_count) {                  // warp-uniform
+            if (lane == 0) {
+              const long long t0 = p.dbg ? clock64() : 0;
+              if (p.store_ring == 2) tma_store_wait_read_le1();   // tile used 2 stores ago is free
+              else tma_store_wait_read_all();
+              if (p.dbg) c_stw += clock64() - t0;
             }
-          }
-        } else {
-          // ---- fused tf.nn.max_pool (window p.pool, stride 2): stage the whole conv tile
-          // (all channel groups), pool across pixels from smem, store the pooled tile.
-          const bool issuer = tt == 0;
-          if (issuer) {
-            const long long t0 = p.dbg ? clock64() : 0;
-            tma_store_wait_read_all();                    // previous item's pooled tiles are free
-            if (p.dbg) c_stw += clock64() - t0;
-          }
-          asm volatile("bar.sync %0, 128;" ::"r"(1 + dgroup) : "memory");
-          const float ninf = -CUDART_INF_F;
+            __syncwarp();
+            const uint32_t tile_w = out_b + (uint32_t)((dgroup * 4 + q) * (4096 * p.store_ring) +
+                                                       (p.store_ring == 2 ? (n_store & 1) * 4096 : 0));
 #pragma unroll
-          for (int jg = 0; jg < MAX_N / 32; ++jg) {
-            if (jg * 32 < ck.ch_count) {
-              const uint32_t tile_c = out_b + (uint32_t)(dgroup * POOL_STAGE_BYTES + jg * 16384);
-#pragma unroll
-              for (int k = 0; k < 8; ++k) {
-                const int c = jg * 32 + k * 4;
-                const float4 b0 = lds128(par + 4u * (uint32_t)c);
-                float o[4] = {acc[c] + b0.x, acc[c + 1] + b0.y, acc[c + 2] + b0.z,
-                              acc[c + 3] + b0.w};
-                if (affine) {
-                  const float4 s0 = lds128(par + 4u * (uint32_t)(MAX_N + c));
-                  const float4 h0v = lds128(par + 4u * (uint32_t)(2 * MAX_N + c));
-                  o[0] = o[0] * s0.x + h0v.x; o[1] = o[1] * s0.y + h0v.y;
-                  o[2] = o[2] * s0.z + h0v.z; o[3] = o[3] * s0.w + h0v.w;
-                }
-                float4 v;
-                // tf.nn.max_pool ignores cells outside the image: they become -inf
-                v.x = pix_ok ? fmaxf(o[0], lo_clip) : ninf;
-                v.y = pix_ok ? fmaxf(o[1], lo_clip) : ninf;
-                v.z = pix_ok ? fmaxf(o[2], lo_clip) : ninf;
-                v.w = pix_ok ? fmaxf(o[3], lo_clip) : ninf;
-                sts128(tile_c + (uint32_t)(r * 128 + ((k ^ (r & 7)) << 4)), v);
+            for (int k = 0; k < 8; ++k) {
+              const int c = jg * 32 + k * 4;
+              const float4 b0 = lds128(par + 4u * (uint32_t)c);
+              float o[4] = {acc[c] + b0.x, acc[c + 1] + b0.y, acc[c + 2] + b0.z,
+                            acc[c + 3] + b0.w};
+              if (affine) {
+                const float4 s0 = lds128(par + 4u * (uint32_t)(MAX_N + c));
+                const float4 h0v = lds128(par + 4u * (uint32_t)(2 * MAX_N + c));
+                o[0] = o[0] * s0.x + h0v.x; o[1] = o[1] * s0.y + h0v.y;
+                o[2] = o[2] * s0.z + h0v.z; o[3] = o[3] * s0.w + h0v.w;
               }
+              float4 v;
+              v.x = fmaxf(o[0], lo_clip); v.y = fmaxf(o[1], lo_clip);
+              v.z = fmaxf(o[2], lo_clip); v.w = fmaxf(o[3], lo_clip);
+              sts128(tile_w + (uint32_t)(lane * 128 + ((k ^ (lane & 7)) << 4)), v);
             }
-          }
-          asm volatile("bar.sync %0, 128;" ::"r"(1 + dgroup) : "memory");
-          const long long tp0 = p.dbg ? clock64() : 0;
-          // unit = (channel group jg, pooled pixel pp, 16-byte chunk k2); pt_w == 8
-          const int n_pp = p.pt_h * 8;
-          const int n_units = ((ck.ch_count + 31) >> 5) * n_pp * 8;
-          const uint32_t conv_base = out_b + (uint32_t)(dgroup * POOL_STAGE_BYTES);
-          const uint32_t pool_base = conv_base + (uint32_t)(POOL_MAX_GROUPS * 16384);
-          if (p.pool == 3) {
-            for (int u = tt; u < n_units; u += 128)
-              pool_unit<3>(conv_base, pool_base, u, n_pp);
-          } else {
-            for (int u = tt; u < n_units; u += 128)
-              pool_unit<2>(conv_base, pool_base, u, n_pp);
-          }
-          if (p.dbg) c_pool += clock64() - tp0;
-          fence_async_proxy();
-          asm volatile("bar.sync %0, 128;" ::"r"(1 + dgroup) : "memory");
-          if (issuer && tile_valid) {
-            for (int jg = 0; jg * 32 < ck.ch_count; ++jg)
-              tma_store_4d(pool_base + jg * 4096, &p.tmY, ck.y_coff + jg * 32, tw * 8,
-                           th_i * p.pt_h, img);
+            fence_async_proxy();
+            __syncwarp();
+            if (lane == 0)
+              tma_store_4d(tile_w, &p.tmY, ck.y_coff + jg * 32, w0 + q * p.sq_w, h0 + q * p.sq_h, img);
+            ++n_store;
           }
         }
-      } else if (pix_ok && tile_valid) {
+      } else if (pix_ok) {
         float* yrow =
             p.y + (((size_t)img * p.Ho + oh) * p.Wo + ow) * (size_t)p.y_cstride + ck.y_coff;
         // 256-bit stores: each thread writes whole 32-byte sectors of its pixel's channel run.
@@ -762,17 +579,14 @@ conv_tc_kernel(const __grid_constant__ TcParams p) {
       p.dbg[blockIdx.x * 12 + 4] = w_tfull;
       p.dbg[blockIdx.x * 12 + 7] = c_epi;
       p.dbg[blockIdx.x * 12 + 8] = c_stw;
-      p.dbg[blockIdx.x * 12 + 9] = c_pool;
       p.dbg[blockIdx.x * 12 + 10] = c_par;
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (C > 1) cluster_sync_all();           // no CTA leaves while peers may still multicast to it
   if (warp == 1) {
     tc_fence_after();
-    if (TWO) tmem_dealloc_2(tmem_base, (uint32_t)p.tmem_cols);
-    else tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
+    tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
   }
 }
 
@@ -783,8 +597,6 @@ splitk_reduce_kernel(const float* __restrict__ part, float* __restrict__ y,
                      const float* __restrict__ bias, const float* __restrict__ scale,
                      const float* __restrict__ shift, long long npix, int cout, int pitch,
                      int ksplit, int y_cstride, int y_coff, int relu) {
-  pdl_trigger();
-  pdl_wait();
   const int c4n = cout / 4;
   const long long total = npix * c4n;
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
@@ -938,20 +750,12 @@ static int encode_flat_map(CUtensorMap* map, const float* x, long long n, int bo
 
 static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vector<ConvGroup>& groups,
                        int relu, bool has_affine, int y_cstride, const float* x_dev, float* y_dev,
-                       const TcPool* pool, const GatherSpec* gs = nullptr) {
+                       const GatherSpec* gs = nullptr) {
   // A launch made only of 1x1 convs has no spatial structure: walk the B*H*W pixels as one flat
   // row in tiles of 128 consecutive pixels (no ragged image-edge tiles; e.g. 22x76x20 is 262
   // tiles instead of 300, which is two waves of 148 CTAs instead of three).
-  bool flat = !(pool && pool->size > 0) && !gs;
+  bool flat = !gs;
   for (auto& g : groups) flat = flat && g.ksize == 1;
-  {
-    static int env_flat = -1;
-    if (env_flat < 0) {
-      const char* a = getenv("SQDET_TC_FLAT");
-      env_flat = a ? atoi(a) : 1;
-    }
-    if (!env_flat) flat = false;
-  }
   if (flat) {
     W = B * H * W;
     H = 1;
@@ -966,8 +770,7 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
   for (auto& g : groups) maxc = g.Cout > maxc ? g.Cout : maxc;
   int N = 0;
   {
-    const int nmax = (pool && pool->size > 0) ? POOL_MAX_N : MAX_N;
-    const int nsplit = (maxc + nmax - 1) / nmax;
+    const int nsplit = (maxc + MAX_N - 1) / MAX_N;
     N = ((maxc + nsplit - 1) / nsplit + 15) / 16 * 16;
   }
   TcParams& P = im->prm;
@@ -998,41 +801,26 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
   im->bias_total = 0;
   for (auto& g : groups) im->bias_total = (g.bias_base + g.Cout) > im->bias_total ? (g.bias_base + g.Cout) : im->bias_total;
   P.B = B; P.Ho = H; P.Wo = W;                      // stride-1 SAME: output grid == input grid
-  P.ct_h = TILE_H; P.ct_w = TILE_W; P.step_h = TILE_H; P.step_w = TILE_W;
-  P.org_h = P.org_w = 0;
+  P.ct_h = TILE_H; P.ct_w = TILE_W;
   P.tiles_h = (H + TILE_H - 1) / TILE_H;
   P.tiles_w = (W + TILE_W - 1) / TILE_W;
   P.sq_w = 0; P.sq_h = 2;                           // drain warp q stores tile rows 2q, 2q+1
   if (flat) {
-    P.ct_h = 1; P.ct_w = TILE_M; P.step_h = 1; P.step_w = TILE_M;
+    P.ct_h = 1; P.ct_w = TILE_M;
     P.tiles_h = 1; P.tiles_w = (W + TILE_M - 1) / TILE_M;
     P.sq_w = 32; P.sq_h = 0;
   }
-  const bool pooled = pool && pool->size > 0;
   // TMA-store epilogue: needs every chunk to be a whole number of 32-channel groups unless it
   // ends at the tensor's last channel (where the TMA unit clips the tail).
   bool store_ok = (y_cstride % 4 == 0);
-  {
-    static int env_tma = -1;
-    if (env_tma < 0) {
-      const char* a = getenv("SQDET_TC_TMA_STORE");
-      env_tma = a ? atoi(a) : 1;
-    }
-    if (!env_tma) store_ok = false;
-    for (auto& c : im->chunks)
-      if ((c.ch_count % 32) != 0 && (c.y_coff + c.ch_count != y_cstride)) store_ok = false;
-    for (auto& c : im->chunks)
-      if (c.y_coff % 4 != 0) store_ok = false;
-  }
-  if (!store_ok && !pooled && !flat && !gs) {
+  for (auto& c : im->chunks)
+    if ((c.ch_count % 32) != 0 && (c.y_coff + c.ch_count != y_cstride)) store_ok = false;
+  for (auto& c : im->chunks)
+    if (c.y_coff % 4 != 0) store_ok = false;
+  if (!store_ok && !flat && !gs) {
     // Direct-store epilogue: any ct_h x ct_w <= 128 tile works, so pick the shape with the fewest
     // rounds of the persistent grid (ConvDet head on 22x76x20: 8x16 tiles = 900 split-K items =
     // 7 rounds on 148 SMs; 11x11 tiles = 840 items = 6 rounds), then the fewest tiles.
-    static int env_search = -1;
-    if (env_search < 0) {
-      const char* a = getenv("SQDET_TC_TILESEARCH");
-      env_search = a ? atoi(a) : 1;
-    }
     int sms = 148, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1040,7 +828,7 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
     auto rounds_of = [&](long long tiles) { return (tiles * nch + sms - 1) / sms; };
     long long best_tiles = (long long)B * P.tiles_h * P.tiles_w;
     long long best_rounds = rounds_of(best_tiles);
-    for (int th = 1; env_search && th <= 32; ++th) {
+    for (int th = 1; th <= 32; ++th) {
       int twd = TILE_M / th;
       if (twd > 128) twd = 128;
       if (twd < 4) break;
@@ -1048,24 +836,10 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
       const long long rounds = rounds_of(tiles);
       if (rounds < best_rounds || (rounds == best_rounds && tiles < best_tiles * 9 / 10)) {
         best_rounds = rounds; best_tiles = tiles;
-        P.ct_h = th; P.ct_w = twd; P.step_h = th; P.step_w = twd;
+        P.ct_h = th; P.ct_w = twd;
         P.tiles_h = (H + th - 1) / th; P.tiles_w = (W + twd - 1) / twd;
       }
     }
-  }
-  if (pooled) {
-    // conv tile = the conv pixels under a pt_h x pt_w block of stride-2 pooling windows
-    if (pool->size != 2 && pool->size != 3) return 0;
-    P.pool = pool->size;
-    P.pt_h = pool->size == 3 ? 3 : 4;
-    P.pt_w = 8;
-    P.ct_h = 2 * (P.pt_h - 1) + pool->size;      // 7 or 8
-    P.ct_w = 2 * (P.pt_w - 1) + pool->size;      // 17 or 16
-    P.step_h = 2 * P.pt_h; P.step_w = 2 * P.pt_w;
-    P.org_h = pool->pad_t; P.org_w = pool->pad_l;
-    P.Hp = pool->Hp; P.Wp = pool->Wp;
-    P.tiles_h = (pool->Hp + P.pt_h - 1) / P.pt_h;
-    P.tiles_w = (pool->Wp + P.pt_w - 1) / P.pt_w;
   }
   P.kch = kch;
   P.N = N;
@@ -1074,74 +848,32 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
   // error of one conv: 24 -> 4e-7, 48 -> 7e-7, 96 -> 1.3e-6 (fp32 SIMT accumulation: 1e-6 ..
   // 2e-6); 48 is 5% faster end to end than 24 but the truncation bias is systematic, and at
   // 48 the 50-layer ResNet body lands one box coordinate 8e-3 px from the fp32 reference
-  // (the test bar is ~6e-3): 36 keeps the margin.
-  P.seg_stages = (KC == 32) ? 3 : 6;
+  // (the test bar is ~6e-3): 36 keeps the margin.  SQDET_TC_SEG overrides it.
+  static const int env_seg = env_int("SQDET_TC_SEG", 0);
+  P.seg_stages = env_seg > 0 ? env_seg : (KC == 32) ? 3 : 6;
   P.ntiles = B * P.tiles_h * P.tiles_w;
   P.y_cstride = y_cstride;
   P.relu = relu;
   P.lo_row_offset = row;
   P.nchunks = (int)im->chunks.size();
   for (int i = 0; i < P.nchunks; ++i) P.chunk[i] = im->chunks[i];
-  // CTA-pair mode (cta_group::2): needs N % 32 == 0 (2-SM TF32 MMA shape rule) and two tiles
-  static int env_two = -1;
-  if (env_two < 0) {
-    const char* a = getenv("SQDET_TC_2CTA");
-    env_two = a ? atoi(a) : 0;
-  }
-  const bool two_cta = env_two != 0 && (N % 32 == 0) && P.ntiles >= 2;
-  P.two_cta = two_cta ? 1 : 0;
-  {
-    // second splitter warpgroup instead of the second drain group: launches whose MMA stage
-    // (12 MMAs of N/2 clocks) is shorter than the splitter's ~650 clocks AND whose items are K-heavy
-    // (few epilogues per MMA: one drain group keeps up).  Measured (profiles/r2_two_split.txt): ConvDet
-    // 0.280 vs 0.271 ms, fire6/7 +5 %, VGG16 +18 % - the stage is a latency chain, not splitter throughput.
-    static int env_2s = -1;
-    if (env_2s < 0) {
-      const char* a = getenv("SQDET_TC_2SPLIT");
-      env_2s = a ? atoi(a) : 0;   // opt-in (2 = the rule below): measured slower everywhere it applies
-    }
-    int max_iters = 0;
-    for (auto& c : im->chunks)
-      max_iters = (c.tap_count * c.kc_count) > max_iters ? (c.tap_count * c.kc_count) : max_iters;
-    const bool want = env_2s == 1 || (env_2s == 2 && N <= 96 && max_iters >= 24);
-    P.two_split = (want && !two_cta && !pooled && !gs) ? 1 : 0;
-  }
-  const size_t stage = (size_t)TILE_M * KC * 4 + (size_t)2 * (two_cta ? N / 2 : N) * KC * 4;
-  // Pipeline depth and residency: with two CTAs per SM (<= ~110 KB each) there are two
-  // independent TMA->split->MMA->drain pipelines per SM to hide latency; otherwise one deep one.
-  static int env_ctas = -1, env_stages = -1, env_seg = -1;
-  if (env_ctas < 0) {
-    const char* a = getenv("SQDET_TC_CTAS");   env_ctas = a ? atoi(a) : 0;
-    const char* b = getenv("SQDET_TC_STAGES"); env_stages = b ? atoi(b) : 0;
-    const char* c = getenv("SQDET_TC_SEG");    env_seg = c ? atoi(c) : 0;
-  }
-  int ctas = env_ctas > 0 ? env_ctas : 1;   // 384 threads x 168 regs: one CTA per SM
-  static int env_ring = -1;
-  if (env_ring < 0) {
-    const char* a = getenv("SQDET_TC_STORE_RING");
-    env_ring = a ? atoi(a) : 0;
-  }
+  const size_t stage = (size_t)TILE_M * KC * 4 + (size_t)2 * N * KC * 4;
+  // Pipeline depth: as many stages as fit one CTA per SM (512 threads x 128 registers) after the
+  // TMA-store staging; a ring of one staging tile per drain warp instead of two when that buys a
+  // fourth stage.
   auto overhead_for = [&](int ring) {
     return (size_t)(1024 /*alignment*/ + 512 /*barriers*/ + 4 * 3 * MAX_N * 4 /*epilogue params*/ +
-                    1024 + (pooled ? 2 * POOL_STAGE_BYTES : 8 * 4096 * ring) /*store staging*/);
+                    1024 + 8 * 4096 * ring /*store staging*/);
   };
+  const size_t budget = 227 * 1024;
   int ring = 2;
   {
-    const size_t budget = 227 * 1024;
     const int s2 = (int)((budget - overhead_for(2)) / stage), s1 = (int)((budget - overhead_for(1)) / stage);
-    if (env_ring == 1 || (env_ring == 0 && s2 < 4 && s1 > s2)) ring = 1;
+    if (s2 < 4 && s1 > s2) ring = 1;
   }
   P.store_ring = ring;
   const size_t overhead = overhead_for(ring);
-  int stages = 0;
-  for (; ctas >= 1; --ctas) {
-    const size_t budget = (ctas == 1 ? 227 * 1024 : (227 * 1024) / ctas - 1024) - overhead;
-    stages = (int)(budget / stage);
-    if (stages >= 3 || ctas == 1) break;
-  }
-  if (ctas < 1) ctas = 1;
-  const int max_stages = env_stages > 0 ? env_stages : MAX_STAGES;
-  if (stages > max_stages) stages = max_stages;
+  int stages = (int)((budget - overhead) / stage);
   if (stages > MAX_STAGES) stages = MAX_STAGES;
   // TMEM: two accumulator buffers (2N columns) + one [a_hi | a_lo] slot (2*KC columns) per stage
   while (stages > 2 && 2 * N + stages * 2 * KC > 512) --stages;
@@ -1152,78 +884,49 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
     while (cols < 2 * N + stages * 2 * KC) cols <<= 1;
     P.tmem_cols = cols;
   }
-  if (env_seg > 0) P.seg_stages = env_seg;
-  {
-    static float env_comp = -1.f;
-    if (env_comp < 0.f) {
-      const char* a = getenv("SQDET_TC_BIAS_COMP");
-      env_comp = a ? (float)atof(a) : 1.4e-8f;
-    }
-    P.bias_comp = env_comp;
-  }
-  {
-    const char* a = getenv("SQDET_TC_ABLATE");
-    P.ablate = a ? atoi(a) : 0;
-  }
+  static const float env_comp = env_float("SQDET_TC_BIAS_COMP", 1.4e-8f);
+  P.bias_comp = env_comp;
   im->smem_bytes = stages * stage + overhead;
   {
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    // Cluster size for the weight multicast: 2 packs all 148 SMs (74 TPC pairs); 4 quarters the
-    // L2->SM weight traffic but strands SMs of GPCs whose SM count is not a multiple of 4.
-    static int env_cluster = -1;
-    if (env_cluster < 0) {
-      const char* a = getenv("SQDET_TC_CLUSTER");
-      env_cluster = a ? atoi(a) : 1;   // measured: multicast (2, 4) is slower, see DESIGN.md
-    }
-    int cluster = (env_cluster == 4 || env_cluster == 2) ? env_cluster : 1;
-    if (P.two_cta) cluster = 2;
-    if (P.ntiles < cluster) cluster = 1;
-    P.cluster = cluster;
-    const long long supers = (long long)((P.ntiles + cluster - 1) / cluster) * P.nchunks;
-    long long nclusters = (long long)(sms * ctas) / cluster;
-    if (supers < nclusters) nclusters = supers;
-    im->grid = dim3((unsigned)(nclusters * cluster));
+    const long long items = (long long)P.ntiles * P.nchunks;
+    const long long nctas = items < sms ? items : sms;
+    im->grid = dim3((unsigned)nctas);
     // Static longest-processing-time-first schedule when chunks differ in cost (a fire expand
     // pair: 1x1 items of kch stages, 3x3 items of 9*kch): round-robin leaves e.g. 12 of 148 CTAs
     // with 7 expensive items against 6 (207 vs 182 stages on fire10); LPT hands those CTAs
     // fewer cheap items instead.
-    static int env_lpt = -1;
-    if (env_lpt < 0) {
-      const char* a = getenv("SQDET_TC_LPT");
-      env_lpt = a ? atoi(a) : 1;
-    }
     bool differ = false;
     for (auto& c : im->chunks)
       if (c.tap_count * c.kc_count != im->chunks[0].tap_count * im->chunks[0].kc_count) differ = true;
     // (only when a CTA gets few items: with dozens per CTA round-robin is already balanced, and
     // keeping a tile's 1x1 and 3x3 items adjacent in time is better for L2 - measured on fire2/3)
-    if (env_lpt && differ && supers > nclusters && supers < 24 * nclusters) {
-      const int spc_h = (P.ntiles + cluster - 1) / cluster;
+    if (differ && items > nctas && items < 24 * nctas) {
       std::vector<int> order(im->chunks.size());
       for (size_t i = 0; i < order.size(); ++i) order[i] = (int)i;
       auto cost_of = [&](int c) { return 2 * im->chunks[c].tap_count * im->chunks[c].kc_count + 3; };   // + epilogue
       std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return cost_of(a) > cost_of(b); });
-      typedef std::pair<long long, int> Bin;     // (load, cluster id): least loaded first
+      typedef std::pair<long long, int> Bin;     // (load, CTA id): least loaded first
       std::priority_queue<Bin, std::vector<Bin>, std::greater<Bin>> heap;
-      for (int b = 0; b < (int)nclusters; ++b) heap.push(Bin(0, b));
-      std::vector<std::vector<int>> lists((size_t)nclusters);
+      for (int b = 0; b < (int)nctas; ++b) heap.push(Bin(0, b));
+      std::vector<std::vector<int>> lists((size_t)nctas);
       for (int c : order)
-        for (int t = 0; t < spc_h; ++t) {
+        for (int t = 0; t < P.ntiles; ++t) {
           Bin b = heap.top();
           heap.pop();
-          lists[(size_t)b.second].push_back(c * spc_h + t);
+          lists[(size_t)b.second].push_back(c * P.ntiles + t);
           b.first += cost_of(c);
           heap.push(b);
         }
-      std::vector<int> sched((size_t)nclusters + 1);
-      int pos = (int)nclusters + 1;
-      for (int b = 0; b < (int)nclusters; ++b) {
+      std::vector<int> sched((size_t)nctas + 1);
+      int pos = (int)nctas + 1;
+      for (int b = 0; b < (int)nctas; ++b) {
         sched[(size_t)b] = pos;
         pos += (int)lists[(size_t)b].size();
       }
-      sched[(size_t)nclusters] = pos;
+      sched[(size_t)nctas] = pos;
       for (auto& l : lists) sched.insert(sched.end(), l.begin(), l.end());
       SQ_CUDA(cudaMalloc(&im->d_sched, sizeof(int) * sched.size()));
       SQ_CUDA(cudaMemcpy(im->d_sched, sched.data(), sizeof(int) * sched.size(), cudaMemcpyHostToDevice));
@@ -1261,40 +964,25 @@ static int plan_common(TcImpl* im, int B, int H, int W, int Cin, const std::vect
     rc = encode_act_map(&P.tmA, x_dev, B, H, W, Cin, KC, P.ct_w, P.ct_h);
     if (rc) return rc;
   }
-  {
-    const bool ok = store_ok;
-    if (pooled && !ok) return 0;          // the fused pool exists only on the TMA-store path
-    if (ok) {
-      if (pooled)
-        rc = encode_act_map(&P.tmY, y_dev, B, pool->Hp, pool->Wp, y_cstride, 32, P.pt_w, P.pt_h);
-      else
-        rc = flat ? encode_act_map(&P.tmY, y_dev, B, H, W, y_cstride, 32, 32, 1)
-                  : encode_act_map(&P.tmY, y_dev, B, H, W, y_cstride, 32, TILE_W, 2);   // per-warp rows
-      if (rc) return rc;
-    }
-    P.tma_store = ok ? 1 : 0;
-  }
-  rc = encode_w_map(&P.tmW, im->d_w, row * 2, KC, N);
-  if (rc) return rc;
-  if (P.cluster > 1) {
-    rc = encode_w_map(&P.tmWs, im->d_w, row * 2, KC, P.two_cta ? N / 2 : 2 * N / P.cluster);
+  if (store_ok) {
+    rc = flat ? encode_act_map(&P.tmY, y_dev, B, H, W, y_cstride, 32, 32, 1)
+              : encode_act_map(&P.tmY, y_dev, B, H, W, y_cstride, 32, TILE_W, 2);   // per-warp rows
     if (rc) return rc;
   }
+  P.tma_store = store_ok ? 1 : 0;
+  rc = encode_w_map(&P.tmW, im->d_w, row * 2, KC, N);
+  if (rc) return rc;
   // opt in to the full 227 KB once per DEVICE for every instantiation (the attribute is per
   // function and per device context, not per launch, so it must cover the largest plan)
   static unsigned long long attr_devs = 0ull;
   int attr_dev = 0;
   SQ_CUDA(cudaGetDevice(&attr_dev));
   if (attr_dev >= 64 || !((attr_devs >> attr_dev) & 1ull)) {
-    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<32, false, false>,
+    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<32, false>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<16, false, false>,
+    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<16, false>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<32, true, false>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<16, true, false>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
-    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<32, false, true>,
+    SQ_CUDA(cudaFuncSetAttribute(conv_tc_kernel<32, true>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 232448));
     if (attr_dev < 64) attr_devs |= 1ull << attr_dev;
   }
@@ -1332,11 +1020,7 @@ static int launch_impl(const TcImpl* im, const float* x_dev, float* y_dev, cudaS
   // the tensor map bakes in the activation address the plan was made for
   (void)x_dev;
   (void)y_dev;
-  static int debug = -1;
-  if (debug < 0) {
-    const char* d = getenv("SQDET_TC_DEBUG");
-    debug = d ? atoi(d) : 0;
-  }
+  static const int debug = env_int("SQDET_TC_DEBUG", 0);
   TcParams prm = im->prm;
   if (prm.gather && x_dev) {
     bool found = false;
@@ -1351,14 +1035,6 @@ static int launch_impl(const TcImpl* im, const float* x_dev, float* y_dev, cudaS
       prm.tmX = m;
     }
   }
-  {
-    static int exp_mode = -1;
-    if (exp_mode < 0) {
-      const char* x = getenv("SQDET_TC_EXP");
-      exp_mode = x ? atoi(x) : 0;
-    }
-    prm.exp_mode = exp_mode;
-  }
   long long* dbg = nullptr;
   const int nb = (int)im->grid.x;
   if (debug) {
@@ -1366,39 +1042,15 @@ static int launch_impl(const TcImpl* im, const float* x_dev, float* y_dev, cudaS
     SQ_CUDA(cudaMemsetAsync(dbg, 0, sizeof(long long) * 12 * nb, stream));
     prm.dbg = dbg;
   }
-  if (prm.cluster <= 1) {
-    // classic launch (no cluster attribute: keeps the non-cluster CTA->SM placement path)
-    if (prm.gather)
-      SQ_CUDA(launch_kernel(conv_tc_kernel<32, false, true>, im->grid, dim3(NUM_THREADS), im->smem_bytes,
-                            stream, prm));
-    else if (im->KC == 32)
-      SQ_CUDA(launch_kernel(conv_tc_kernel<32, false, false>, im->grid, dim3(NUM_THREADS), im->smem_bytes,
-                            stream, prm));
-    else
-      SQ_CUDA(launch_kernel(conv_tc_kernel<16, false, false>, im->grid, dim3(NUM_THREADS), im->smem_bytes,
-                            stream, prm));
-  } else {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = im->grid;
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = im->smem_bytes;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)prm.cluster;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t le;
-    if (prm.two_cta)
-      le = (im->KC == 32) ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<32, true, false>, prm)
-                          : cudaLaunchKernelEx(&cfg, conv_tc_kernel<16, true, false>, prm);
-    else
-      le = (im->KC == 32) ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<32, false, false>, prm)
-                          : cudaLaunchKernelEx(&cfg, conv_tc_kernel<16, false, false>, prm);
-    if (le != cudaSuccess) return cuda_fail(le, "cudaLaunchKernelEx(conv_tc_kernel)");
-  }
+  if (prm.gather)
+    SQ_CUDA(launch_kernel(conv_tc_kernel<32, true>, im->grid, dim3(NUM_THREADS), im->smem_bytes, stream,
+                          prm));
+  else if (im->KC == 32)
+    SQ_CUDA(launch_kernel(conv_tc_kernel<32, false>, im->grid, dim3(NUM_THREADS), im->smem_bytes, stream,
+                          prm));
+  else
+    SQ_CUDA(launch_kernel(conv_tc_kernel<16, false>, im->grid, dim3(NUM_THREADS), im->smem_bytes, stream,
+                          prm));
   SQ_CHECK_LAUNCH("conv_tc_kernel");
   if (im->ksplit > 1) {
     const long long total = im->npix * (im->cout / 4);
@@ -1419,11 +1071,11 @@ static int launch_impl(const TcImpl* im, const float* x_dev, float* y_dev, cudaS
     for (int b = 0; b < nb; ++b)
       for (int k = 0; k < 12; ++k) a[k] += (double)h[(size_t)b * 12 + k] / nb;
     fprintf(stderr,
-            "[tc] grid %d tile %dx%d ntiles %d%s cluster %d%s smem %zu KC %d N %d kch %d chunks %d stages %d seg %d | per-CTA avg cycles: "
+            "[tc] grid %d tile %dx%d ntiles %d%s smem %zu KC %d N %d kch %d chunks %d stages %d seg %d | per-CTA avg cycles: "
             "total %.0f stages %.0f | waits: producer(empty) %.0f mma(split) %.0f mma(tempty) %.0f "
-            "splitter(full) %.0f drain(tfull) %.0f | epilogue %.0f (store-wait %.0f, pool %.0f, params %.0f)\n",
-            nb, prm.ct_h, prm.ct_w, prm.ntiles, prm.sched ? " LPT" : "", prm.cluster, prm.two_cta ? " (cta_group::2)" : "", im->smem_bytes, im->KC, prm.N, prm.kch, prm.nchunks, prm.stages, prm.seg_stages,
-            a[5], a[6], a[0], a[1], a[2], a[3], a[4], a[7], a[8], a[9], a[10]);
+            "splitter(full) %.0f drain(tfull) %.0f | epilogue %.0f (store-wait %.0f, params %.0f)\n",
+            nb, prm.ct_h, prm.ct_w, prm.ntiles, prm.sched ? " LPT" : "", im->smem_bytes, im->KC, prm.N, prm.kch, prm.nchunks, prm.stages, prm.seg_stages,
+            a[5], a[6], a[0], a[1], a[2], a[3], a[4], a[7], a[8], a[10]);
   }
   return SQDET_OK;
 }
@@ -1463,38 +1115,13 @@ bool tc_conv_eligible(int Cin, int Cout, int size, int stride, int padding, int 
   return true;
 }
 
-bool tc_pool_fusable(const int* couts, const int* coffs, int ngroups, int y_cstride, int pool_size,
-                     int pool_stride) {
-  // mirrors plan_common: uniform chunk width N; every chunk must be whole 32-channel groups
-  // unless it ends the output tensor (TMA clips the tail there)
-  if ((pool_size != 2 && pool_size != 3) || pool_stride != 2 || (y_cstride % 4)) return false;
-  int maxc = 0;
-  for (int g = 0; g < ngroups; ++g) maxc = couts[g] > maxc ? couts[g] : maxc;
-  const int nsplit = (maxc + POOL_MAX_N - 1) / POOL_MAX_N;
-  const int N = ((maxc + nsplit - 1) / nsplit + 15) / 16 * 16;
-  int nchunks = 0;
-  for (int g = 0; g < ngroups; ++g)
-    for (int cb = 0; cb < couts[g]; cb += N, ++nchunks) {
-      const int cnt = (couts[g] - cb) < N ? (couts[g] - cb) : N;
-      if ((cnt % 32) != 0 && (coffs[g] + cb + cnt != y_cstride)) return false;
-      if ((coffs[g] + cb) % 4) return false;
-    }
-  return nchunks <= MAX_CHUNKS;
-}
-
 int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int size, int stride,
                  int padding, int relu, bool has_affine, int y_cstride, int y_coff,
-                 const float* x_dev, float* y_dev, const TcPool* pool) {
+                 const float* x_dev, float* y_dev) {
   plan->enabled = false;
   // First layer: 3x3 conv over a 3-channel image (stride 1 or 2, SAME or VALID) -> gather mode
   if (Cin == 3 && size == 3 && (stride == 1 || stride == 2) && (Cout % 4) == 0 &&
       (y_cstride % 4) == 0 && (y_coff % 4) == 0) {
-    static int env_gather = -1;
-    if (env_gather < 0) {
-      const char* a = getenv("SQDET_TC_GATHER");
-      env_gather = a ? atoi(a) : 1;
-    }
-    if (!env_gather) return 0;
     const Geom gh = tf_geometry(H, size, stride, padding);
     const Geom gw = tf_geometry(W, size, stride, padding);
     if (gh.out <= 0 || gw.out <= 0) return 0;
@@ -1502,7 +1129,7 @@ int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int s
     GatherSpec gs{B, H, W, stride, gh.pad_before, gw.pad_before};
     std::vector<ConvGroup> groups = {{1, Cout, y_coff, 0}};   // one K block of 32 (27 real taps)
     int rc = plan_common(im, B, gh.out, gw.out, 32, groups, relu, has_affine, y_cstride, x_dev,
-                         y_dev, pool, &gs);
+                         y_dev, &gs);
     if (rc <= 0) {
       void* p = im;
       release_impl(&p);
@@ -1525,24 +1152,19 @@ int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int s
   // three partial convs over the filter rows, then a deterministic reduction.
   int ksplit = 1;
   {
-    static int env_split = -1;
-    if (env_split < 0) {
-      const char* a = getenv("SQDET_TC_SPLITK");
-      env_split = a ? atoi(a) : 1;
-    }
     int sms = 148, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const long long ntiles = (long long)B * ((H + TILE_H - 1) / TILE_H) * ((W + TILE_W - 1) / TILE_W);
     const bool few_items = Cout <= MAX_N && ntiles < 4LL * sms && (ntiles % sms) != 0 &&
                            (double)(ntiles % sms) / sms < 0.5;
-    if (env_split && !pool && size == 3 && few_items && Cin >= 96 && (Cout % 4) == 0) ksplit = 3;
+    if (size == 3 && few_items && Cin >= 96 && (Cout % 4) == 0) ksplit = 3;
   }
   std::vector<ConvGroup> groups;
   int rc;
   if (ksplit == 1) {
     groups = {{size, Cout, y_coff, 0}};
-    rc = plan_common(im, B, H, W, Cin, groups, relu, has_affine, y_cstride, x_dev, y_dev, pool);
+    rc = plan_common(im, B, H, W, Cin, groups, relu, has_affine, y_cstride, x_dev, y_dev);
   } else {
     const int pitch = (Cout + 7) / 8 * 8;
     im->ksplit = ksplit;
@@ -1558,15 +1180,10 @@ int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int s
       delete im;
       return cuda_fail(ce, "cudaMalloc(split-K scratch)");
     }
-    static int env_rows = -1;
-    if (env_rows < 0) {
-      const char* a = getenv("SQDET_TC_SPLITK_ROWS");
-      env_rows = a ? atoi(a) : 0;
-    }
     const int KCs = (Cin % 32 == 0) ? 32 : 16, kch_all = Cin / KCs;
     for (int s2 = 0; s2 < ksplit; ++s2) {
       ConvGroup g{size, Cout, s2 * pitch, 0};
-      if (env_rows || kch_all % ksplit != 0) {
+      if (kch_all % ksplit != 0) {
         g.tap_begin = s2 * size;         // one filter row per partial (reads the input ksplit times)
         g.tap_count = size;
       } else {
@@ -1576,8 +1193,7 @@ int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int s
       groups.push_back(g);
     }
     // partials: no bias / affine / relu in the conv epilogue (they are applied by the reduction)
-    rc = plan_common(im, B, H, W, Cin, groups, 0, has_affine, ksplit * pitch, x_dev, im->d_scratch,
-                     nullptr);
+    rc = plan_common(im, B, H, W, Cin, groups, 0, has_affine, ksplit * pitch, x_dev, im->d_scratch);
     if (rc > 0) im->prm.bias = nullptr, im->prm.scale = nullptr, im->prm.shift = nullptr;
   }
   if (rc <= 0) {
@@ -1595,12 +1211,12 @@ int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int s
 }
 
 int tc_fire_plan(TcFirePlan* plan, int B, int H, int W, int S, int E1, int E3, const float* q_dev,
-                 float* y_dev, const TcPool* pool) {
+                 float* y_dev) {
   plan->enabled = false;
   if (S % 16 != 0 || S < 16 || (E1 % 4) || (E3 % 4)) return 0;
   TcImpl* im = new TcImpl();
   std::vector<ConvGroup> groups = {{1, E1, 0, 0}, {3, E3, E1, E1}};
-  int rc = plan_common(im, B, H, W, S, groups, 1, false, E1 + E3, q_dev, y_dev, pool);
+  int rc = plan_common(im, B, H, W, S, groups, 1, false, E1 + E3, q_dev, y_dev);
   if (rc <= 0) {
     void* p = im;
     release_impl(&p);
@@ -1642,17 +1258,6 @@ int tc_fire_pack_weights(TcFirePlan* plan, const float* w_e1, const float* b_e1,
   return SQDET_OK;
 }
 
-int launch_splitk_reduce(const float* part, float* y, const float* bias, const float* scale,
-                         const float* shift, long long npix, int cout, int pitch, int ksplit,
-                         int y_cstride, int y_coff, int relu, cudaStream_t stream) {
-  const long long total = npix * (cout / 4);
-  long long blocks = (total + 255) / 256;
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  SQ_CUDA(launch_kernel(splitk_reduce_kernel, dim3((unsigned)blocks), dim3(256), 0, stream, part, y, bias,
-                        scale, shift, npix, cout, pitch, ksplit, y_cstride, y_coff, relu));
-  return SQDET_OK;
-}
-
 int launch_conv_tc(const TcConvPlan& plan, const float* x_dev, float* y_dev, cudaStream_t stream) {
   return launch_impl(static_cast<const TcImpl*>(plan.impl), x_dev, y_dev, stream);
 }
@@ -1677,7 +1282,7 @@ int conv2d_tc_oneshot(const float* x_dev, const float* w_hwio_dev, const float* 
                       int y_cstride, int y_coff, cudaStream_t stream) {
   TcConvPlan plan;
   int rc = tc_conv_plan(&plan, B, H, W, Cin, Cout, size, stride, padding, relu,
-                        scale_dev != nullptr, y_cstride, y_coff, x_dev, y_dev, nullptr);
+                        scale_dev != nullptr, y_cstride, y_coff, x_dev, y_dev);
   if (rc < 0) return rc;
   if (rc == 0) {
     // shape not taken by the tensor-core path (e.g. conv1, Cin = 3): same dispatch as the engine

@@ -24,23 +24,16 @@ struct TcFirePlan {
   void* impl = nullptr;
 };
 
-// A stride-2 max-pool (window 2 or 3) fused into the conv's epilogue: the conv output is never
-// written; y is the POOLED tensor [B, Hp, Wp, C].  pad_* are tf.nn.max_pool's pad_before.
-struct TcPool {
-  int size = 0, pad_t = 0, pad_l = 0, Hp = 0, Wp = 0;
-};
 bool tc_conv_eligible(int Cin, int Cout, int size, int stride, int padding, int y_cstride,
                       int y_coff);
-bool tc_pool_fusable(const int* couts, const int* coffs, int ngroups, int y_cstride, int pool_size,
-                     int pool_stride);
 
 // Returns 1 when the shape is taken by the tensor-core path (plan->enabled), 0 when it is
 // left to the fp32 SIMT kernel, negative on error.
 int tc_conv_plan(TcConvPlan* plan, int B, int H, int W, int Cin, int Cout, int size, int stride,
                  int padding, int relu, bool has_affine, int y_cstride, int y_coff,
-                 const float* x_dev, float* y_dev, const TcPool* pool);
+                 const float* x_dev, float* y_dev);
 int tc_fire_plan(TcFirePlan* plan, int B, int H, int W, int S, int E1, int E3,
-                 const float* q_dev, float* y_dev, const TcPool* pool);
+                 const float* q_dev, float* y_dev);
 int tc_conv_pack_weights(TcConvPlan* plan, const float* w_hwio, const float* bias);
 int tc_conv_set_affine(TcConvPlan* plan, const float* scale, const float* shift);
 int tc_fire_pack_weights(TcFirePlan* plan, const float* w_e1, const float* b_e1,

@@ -23,7 +23,6 @@
 #include "common.cuh"
 #include "conv_tc.cuh"
 #include "fire_tc.cuh"
-#include "halo_tc.cuh"
 #include "first_tc.cuh"
 
 namespace sqdet {
@@ -33,9 +32,6 @@ static thread_local std::string g_last_error;
 
 void set_error(const std::string& msg) { g_last_error = msg; }
 
-static thread_local bool g_pdl_launch = false;
-void set_pdl_launch(bool on) { g_pdl_launch = on; }
-bool pdl_launch() { return g_pdl_launch; }
 int fail(int code, const std::string& msg) {
   g_last_error = msg;
   return code;
@@ -78,7 +74,6 @@ struct ConvSpec {
   float* scale = nullptr;      // device, BN only
   float* shift = nullptr;
   TcConvPlan tc;               // tensor-core plan (valid when tc.enabled)
-  HaloConvPlan halo;           // halo-tile 3x3 plan (valid when halo.enabled; then tc is not planned)
 };
 
 struct Op {
@@ -93,7 +88,7 @@ struct Op {
   FusedFirePlan fused;           // whole fire module in one kernel (valid when fused.enabled)
   FirstTcPlan first_tc;          // first layer conv+pool on tcgen05 (valid when first_tc.enabled)
   bool skip = false;             // pool op whose work happens in the producer's epilogue
-  int fused_pool_op = -1;        // index of the pool op fused into this conv / fire
+  int fused_pool_op = -1;        // index of the pool op fused into this first layer
   bool first_layer_fused = false;  // Cin=3 stride-2 conv + 3x3/2 pool as one FFMA kernel
   int out = -1;                  // tensor actually written (dst, or the fused pool's dst)
 };
@@ -249,7 +244,6 @@ static int run_conv(sqdet_engine* e, const ConvSpec& c, const float* x_override,
   const Tensor& in = e->tensors[c.src];
   const Tensor& out = e->tensors[c.dst];
   const float* x = (c.src == 0 && x_override) ? x_override : in.dev;
-  if (c.halo.enabled) return launch_halo_conv(c.halo, stream);
   if (c.tc.enabled) return launch_conv_tc(c.tc, x, out.dev, stream);
   ConvArgs a;
   a.x = x;
@@ -275,7 +269,6 @@ static int run_op(sqdet_engine* e, const Op& op, const float* x_override, cudaSt
         const Tensor& in = e->tensors[c.src];
         const float* x = (c.src == 0 && x_override) ? x_override : in.dev;
         if (op.first_tc.enabled) return launch_first_tc(op.first_tc, x, stream);
-        if (c.tc.enabled) return launch_conv_tc(c.tc, x, e->tensors[op.out].dev, stream);
         return launch_conv_pool_simt(x, e->params[c.p_kernel].dev,
                                      c.p_bias >= 0 ? e->params[c.p_bias].dev : nullptr, c.scale,
                                      c.shift, e->tensors[op.out].dev, in.B, in.H, in.W, c.Cout,
@@ -322,7 +315,7 @@ struct NcclApi {
 static NcclApi g_nccl;
 static int nccl_load() {
   if (g_nccl.handle) return SQDET_OK;
-  const char* env = getenv("SQDET_NCCL_LIB");
+  static const char* const env = env_str("SQDET_NCCL_LIB");
   const char* cands[] = {env, "libnccl.so.2", "libnccl.so"};
   void* h = nullptr;
   for (const char* c : cands) {
@@ -409,10 +402,6 @@ static int prepare_params(sqdet_engine* e) {
           int rc = tc_conv_set_affine(&c.tc, sc.data(), sh.data());
           if (rc) return rc;
         }
-        if (c.halo.enabled) {
-          int rc = halo_conv_set_affine(&c.halo, sc.data(), sh.data());
-          if (rc) return rc;
-        }
         if (op.first_tc.enabled && &c == &op.convs[0]) {
           int rc = first_tc_set_affine(&op.first_tc, sc.data(), sh.data());
           if (rc) return rc;
@@ -430,10 +419,6 @@ static int prepare_params(sqdet_engine* e) {
     }
     for (auto& c : op.convs) {
       const float* bias = c.p_bias >= 0 ? e->params[c.p_bias].host.data() : nullptr;
-      if (c.halo.enabled) {
-        int rc = halo_conv_pack_weights(&c.halo, e->params[c.p_kernel].host.data(), bias);
-        if (rc) return rc;
-      }
       if (!c.tc.enabled) continue;
       int rc = tc_conv_pack_weights(&c.tc, e->params[c.p_kernel].host.data(), bias);
       if (rc) return rc;
@@ -477,28 +462,11 @@ static void drop_graph(sqdet_engine* e) {
 }
 
 static int enqueue_all(sqdet_engine* e, const float* images_dev, cudaStream_t stream) {
-  // Programmatic dependent launch for every kernel after the first (whose input comes from a
-  // copy or from the caller): see common.cuh.  Opt-in (SQDET_PDL=1): measured on the captured
-  // forward graph it changes nothing (1.916 vs 1.912 ms/step, profiles/r2_pdl.txt) - the graph
-  // already removes the launch gaps and the kernels' prologues are ~2 us of a 1.9 ms step.
-  static int env_pdl = -1;
-  if (env_pdl < 0) {
-    const char* a = getenv("SQDET_PDL");
-    env_pdl = a ? atoi(a) : 0;
-  }
-  int rc = SQDET_OK;
-  bool first = true;
   for (const auto& op : e->ops) {
-    rc = run_op(e, op, images_dev, stream);
-    if (rc) break;
-    if (first && !op.skip) {
-      first = false;
-      set_pdl_launch(env_pdl != 0);
-    }
+    int rc = run_op(e, op, images_dev, stream);
+    if (rc) return rc;
   }
-  if (!rc) rc = run_postproc(e, stream);
-  set_pdl_launch(false);
-  return rc;
+  return run_postproc(e, stream);
 }
 
 static int forward_impl(sqdet_engine* e, const float* images_dev, cudaStream_t stream) {
@@ -598,7 +566,6 @@ int sqdet_destroy(sqdet_engine* e) {
       if (c.scale) cudaFree(c.scale);
       if (c.shift) cudaFree(c.shift);
       tc_conv_release(&c.tc);
-      halo_conv_release(&c.halo);
     }
     tc_fire_release(&op.tcfire);
     fused_fire_release(&op.fused);
@@ -790,80 +757,28 @@ int sqdet_finalize(sqdet_engine* e) {
     return fail(SQDET_ERR_INVALID_ARG, "max_dets smaller than TOP_N_DETECTION");
   if (topn && c.top_n_detection > 1024)
     return fail(SQDET_ERR_UNSUPPORTED, "TOP_N_DETECTION above 1024 is not supported");
-  // Pool fusion: a stride-2 max-pool whose input is produced by a tensor-core conv / fire and
-  // read by nobody else runs inside that producer's epilogue; the un-pooled tensor is never
-  // materialised (for SqueezeDet: fire3+pool3, fire5+pool5).
+  // First layer: a Cin = 3, stride-2 conv followed by a 3x3/2 max-pool that nobody else reads runs
+  // as one kernel (both math modes); the un-pooled tensor is never materialised.
   for (auto& op : e->ops) op.out = op.dst;
-  {
-    static int env_fuse = -1;
-    if (env_fuse < 0) {
-      const char* a = getenv("SQDET_FUSE_POOL");
-      env_fuse = a ? atoi(a) : 1;
+  for (int i = 0; i + 1 < (int)e->ops.size(); ++i) {
+    Op& prod = e->ops[i];
+    Op& pool = e->ops[i + 1];
+    if (prod.kind != OP_CONV || pool.kind != OP_POOL || pool.src != prod.dst) continue;
+    const ConvSpec& cs = prod.convs[0];
+    if (!conv_pool_simt_eligible(cs.Cin, cs.Cout, cs.size, cs.stride, pool.size, pool.stride))
+      continue;
+    int readers = 0;
+    for (const auto& o : e->ops) {
+      if (o.src == prod.dst || o.src2 == prod.dst) ++readers;
+      for (const auto& c2 : o.convs)
+        if (&o != &prod && c2.src == prod.dst) ++readers;
     }
-    const int nops = (int)e->ops.size();
-    // first layer: Cin = 3, stride-2 conv + 3x3/2 pool -> one FFMA kernel (both math modes)
-    for (int i = 0; env_fuse && i + 1 < nops; ++i) {
-      Op& prod = e->ops[i];
-      Op& pool = e->ops[i + 1];
-      if (prod.kind != OP_CONV || pool.kind != OP_POOL || pool.src != prod.dst) continue;
-      const ConvSpec& cs = prod.convs[0];
-      if (!conv_pool_simt_eligible(cs.Cin, cs.Cout, cs.size, cs.stride, pool.size, pool.stride))
-        continue;
-      int readers = 0;
-      for (const auto& o : e->ops) {
-        if (o.src == prod.dst || o.src2 == prod.dst) ++readers;
-        for (const auto& c2 : o.convs)
-          if (&o != &prod && c2.src == prod.dst) ++readers;
-      }
-      if (readers != 1 || prod.dst == e->preds) continue;
-      prod.first_layer_fused = true;
-      prod.fused_pool_op = i + 1;
-      prod.out = pool.dst;
-      pool.skip = true;
-      e->tensors[prod.dst].materialized = false;
-    }
-    // Tensor-core conv/fire + pool fusion is implemented and parity-green but currently a net
-    // loss (the pooled epilogue saturates the drain warps: fire3+pool3 0.43 ms fused vs 0.36 ms
-    // unfused), so it is opt-in (SQDET_FUSE_TC_POOL=1) until the pooling moves to its own warps.
-    static int env_tc_pool = -1;
-    if (env_tc_pool < 0) {
-      const char* a = getenv("SQDET_FUSE_TC_POOL");
-      env_tc_pool = a ? atoi(a) : 0;
-    }
-    for (int i = 0; env_fuse && env_tc_pool && c.math_mode == SQDET_MATH_TF32X3_TC && i + 1 < nops; ++i) {
-      Op& prod = e->ops[i];
-      Op& pool = e->ops[i + 1];
-      if (pool.kind != OP_POOL || pool.src != prod.dst || pool.skip) continue;
-      if (prod.kind != OP_CONV && prod.kind != OP_FIRE) continue;
-      if (prod.dst == e->preds) continue;
-      int readers = 0;
-      for (const auto& o : e->ops) {
-        if (o.src == prod.dst || o.src2 == prod.dst) ++readers;
-        for (const auto& cs : o.convs)
-          if (&o != &prod && cs.src == prod.dst) ++readers;
-      }
-      if (readers != 1) continue;
-      const Tensor& pt = e->tensors[prod.dst];
-      bool ok = false;
-      if (prod.kind == OP_CONV) {
-        const ConvSpec& cs = prod.convs[0];
-        int couts[1] = {cs.Cout}, coffs[1] = {0};
-        ok = tc_conv_eligible(cs.Cin, cs.Cout, cs.size, cs.stride, cs.padding, pt.C, 0) &&
-             tc_pool_fusable(couts, coffs, 1, pt.C, pool.size, pool.stride);
-      } else {
-        const ConvSpec& sq = prod.convs[0];
-        int couts[2] = {prod.convs[1].Cout, prod.convs[2].Cout};
-        int coffs[2] = {0, prod.convs[1].Cout};
-        ok = tc_conv_eligible(sq.Cout, couts[0], 1, 1, SQDET_PAD_SAME, pt.C, 0) &&
-             tc_conv_eligible(sq.Cout, couts[1], 3, 1, SQDET_PAD_SAME, pt.C, coffs[1]) &&
-             tc_pool_fusable(couts, coffs, 2, pt.C, pool.size, pool.stride);
-      }
-      if (!ok) continue;
-      prod.fused_pool_op = i + 1;
-      prod.out = pool.dst;
-      pool.skip = true;
-      e->tensors[prod.dst].materialized = false;
-    }
+    if (readers != 1 || prod.dst == e->preds) continue;
+    prod.first_layer_fused = true;
+    prod.fused_pool_op = i + 1;
+    prod.out = pool.dst;
+    pool.skip = true;
+    e->tensors[prod.dst].materialized = false;
   }
   // activations
   for (size_t i = 0; i < e->tensors.size(); ++i) {
@@ -895,92 +810,27 @@ int sqdet_finalize(sqdet_engine* e) {
     int64_t bytes = 0;
     op.launches = 0;
     if (op.kind == OP_CONV || op.kind == OP_FIRE) {
-      bytes += 4 * e->tensors[op.src].numel() + 4 * e->tensors[op.dst].numel() + 4 * op.params;
-      TcPool pool_spec;
-      const TcPool* pool_ptr = nullptr;
+      bytes = 4 * e->tensors[op.src].numel() + 4 * e->tensors[op.out].numel() + 4 * op.params;
       if (op.first_layer_fused) {
-        bytes = 4 * e->tensors[op.src].numel() + 4 * e->tensors[op.out].numel() + 4 * op.params;
-      }
-      if (op.fused_pool_op >= 0) {
-        const Op& po = e->ops[op.fused_pool_op];
-        const Tensor& un = e->tensors[op.dst];
-        const Geom gh = tf_geometry(un.H, po.size, po.stride, po.padding);
-        const Geom gw = tf_geometry(un.W, po.size, po.stride, po.padding);
-        pool_spec.size = po.size;
-        pool_spec.pad_t = gh.pad_before;
-        pool_spec.pad_l = gw.pad_before;
-        pool_spec.Hp = gh.out;
-        pool_spec.Wp = gw.out;
-        pool_ptr = &pool_spec;
-        bytes = 4 * e->tensors[op.src].numel() + 4 * e->tensors[op.out].numel() + 4 * op.params;
-      }
-      static int env_first_tc = -1;
-      if (env_first_tc < 0) {
-        const char* a = getenv("SQDET_TC_FIRST_POOL");
-        env_first_tc = a ? atoi(a) : 0;
-      }
-      if (c.math_mode == SQDET_MATH_TF32X3_TC && op.first_layer_fused && !env_first_tc) {
-        // first layer on tcgen05, pooled-pixel-major with the pool as a max over accumulators
-        // (first_tc.cu); shapes it declines stay on the fused FFMA kernel
-        ConvSpec& cs = op.convs[0];
-        const Op& po = e->ops[op.fused_pool_op];
-        int rc = first_tc_plan(&op.first_tc, e->tensors[cs.src].B, e->tensors[cs.src].H,
-                               e->tensors[cs.src].W, cs.Cout, cs.size, cs.stride, cs.padding,
-                               cs.relu, cs.p_gamma >= 0, po.size, po.stride, po.padding,
-                               e->tensors[op.out].dev);
-        if (rc < 0) return rc;
-      }
-      if (c.math_mode == SQDET_MATH_TF32X3_TC && op.first_layer_fused && env_first_tc) {
-        // tensor-core first layer (gather mode) with the pool in its epilogue.  Parity-green but
-        // measured slower than the fused FFMA kernel (0.43 ms vs 0.37 ms for SqueezeDet conv1 +
-        // pool1: the pooled epilogue saturates the drain warps), hence opt-in; un-pooled first
-        // layers (VGG16 conv1_1: 0.93 -> 0.36 ms) take the gather mode by default.
-        ConvSpec& cs = op.convs[0];
-        int rc = tc_conv_plan(&cs.tc, e->tensors[cs.src].B, e->tensors[cs.src].H,
-                              e->tensors[cs.src].W, cs.Cin, cs.Cout, cs.size, cs.stride,
-                              cs.padding, cs.relu, cs.p_gamma >= 0, e->tensors[op.out].C,
-                              cs.y_coff, e->tensors[cs.src].dev, e->tensors[op.out].dev, pool_ptr);
-        if (rc < 0) return rc;
-      }
-      if (c.math_mode == SQDET_MATH_TF32X3_TC && !op.first_layer_fused) {
+        if (c.math_mode == SQDET_MATH_TF32X3_TC) {
+          // first layer on tcgen05, pooled-pixel-major with the pool as a max over accumulators
+          // (first_tc.cu); shapes it declines stay on the fused FFMA kernel
+          ConvSpec& cs = op.convs[0];
+          const Op& po = e->ops[op.fused_pool_op];
+          int rc = first_tc_plan(&op.first_tc, e->tensors[cs.src].B, e->tensors[cs.src].H,
+                                 e->tensors[cs.src].W, cs.Cout, cs.size, cs.stride, cs.padding,
+                                 cs.relu, cs.p_gamma >= 0, po.size, po.stride, po.padding,
+                                 e->tensors[op.out].dev);
+          if (rc < 0) return rc;
+        }
+      } else if (c.math_mode == SQDET_MATH_TF32X3_TC) {
         if (op.kind == OP_CONV) {
           ConvSpec& cs = op.convs[0];
-          // 3x3 stride-1 convs on the halo-tile kernel (halo_tc.cu): opt-in.  Measured
-          // (profiles/r2_halo_conv.txt): parity-green, 9x less TMA traffic, but every .ss MMA re-reads
-          // its 4 KB A tile from shared memory, which bounds a thin-N conv at ~86 clocks per MMA -
-          // ConvDet 0.339 vs 0.271 ms, VGG16 / ResNet-50 bodies +14 % / +3 %.  SQDET_HALO_CONV:
-          // 0 never (default), 1 thin heads with few tiles per SM (ConvDet), 2 every shape it takes.
-          static int env_halo = -1;
-          if (env_halo < 0) {
-            const char* a = getenv("SQDET_HALO_CONV");
-            env_halo = a ? atoi(a) : 0;
-          }
-          if (env_halo && !pool_ptr && cs.size == 3 && cs.stride == 1 && cs.padding == SQDET_PAD_SAME &&
-              cs.src != 0) {
-            const Tensor& xin = e->tensors[cs.src];
-            int sms = 148, dev = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            const long long tiles = (long long)xin.B * ((xin.H + 7) / 8) * ((xin.W + 15) / 16);
-            if (env_halo >= 2 || (cs.Cout <= 128 && cs.Cin >= 256 && tiles < 8LL * sms)) {
-              int rch = halo_conv_plan(&cs.halo, xin.B, xin.H, xin.W, cs.Cin, cs.Cout, cs.relu,
-                                       cs.p_gamma >= 0, e->tensors[op.out].C, cs.y_coff, xin.dev,
-                                       e->tensors[op.out].dev);
-              if (rch < 0) return rch;
-            }
-          }
-          if (cs.halo.enabled) {
-            op.launches = cs.halo.launches;
-            op.min_bytes = bytes;
-            continue;
-          }
           int rc = tc_conv_plan(&cs.tc, e->tensors[cs.src].B, e->tensors[cs.src].H,
                                 e->tensors[cs.src].W, cs.Cin, cs.Cout, cs.size, cs.stride,
                                 cs.padding, cs.relu, cs.p_gamma >= 0, e->tensors[op.out].C,
-                                cs.y_coff, e->tensors[cs.src].dev, e->tensors[op.out].dev, pool_ptr);
+                                cs.y_coff, e->tensors[cs.src].dev, e->tensors[op.out].dev);
           if (rc < 0) return rc;
-          if (pool_ptr && rc == 0)
-            return fail(SQDET_ERR_STATE, "pool fusion was promised but the conv plan declined");
         } else {
           ConvSpec& sq = op.convs[0];
           // The whole module as ONE kernel (fire_tc.cu) where it is the faster plan - measured on
@@ -989,12 +839,8 @@ int sqdet_finalize(sqdet_engine* e) {
           // streamed per tile and a 2x squeeze (two M tiles per halo), and lose to the squeeze
           // launch + fused expand pair.  SQDET_FUSED_FIRE: 0 never, 1 this rule, 2 every shape the
           // kernel takes, 3 every shape with >= 4 tiles per SM.
-          static int env_fused = -1;
-          if (env_fused < 0) {
-            const char* a = getenv("SQDET_FUSED_FIRE");
-            env_fused = a ? atoi(a) : 1;
-          }
-          if (env_fused && !pool_ptr && e->tensors[sq.src].dev != nullptr && sq.src != 0) {
+          static const int env_fused = env_int("SQDET_FUSED_FIRE", 1);
+          if (env_fused && e->tensors[sq.src].dev != nullptr && sq.src != 0) {
             const Tensor& xin = e->tensors[sq.src];
             int sms = 148, dev = 0;
             cudaGetDevice(&dev);
@@ -1015,14 +861,12 @@ int sqdet_finalize(sqdet_engine* e) {
           int rc = tc_conv_plan(&sq.tc, e->tensors[sq.src].B, e->tensors[sq.src].H,
                                 e->tensors[sq.src].W, sq.Cin, sq.Cout, 1, 1, SQDET_PAD_SAME, 1,
                                 false, e->tensors[sq.dst].C, 0, e->tensors[sq.src].dev,
-                                e->tensors[sq.dst].dev, nullptr);
+                                e->tensors[sq.dst].dev);
           if (rc < 0) return rc;
           const Tensor& q = e->tensors[sq.dst];
           rc = tc_fire_plan(&op.tcfire, q.B, q.H, q.W, q.C, op.convs[1].Cout, op.convs[2].Cout,
-                            q.dev, e->tensors[op.out].dev, pool_ptr);
+                            q.dev, e->tensors[op.out].dev);
           if (rc < 0) return rc;
-          if (pool_ptr && rc == 0)
-            return fail(SQDET_ERR_STATE, "pool fusion was promised but the fire plan declined");
         }
       }
       if (op.kind == OP_CONV) op.launches = op.convs[0].tc.enabled ? op.convs[0].tc.launches : 1;
@@ -1543,43 +1387,6 @@ int sqdet_conv2d(const float* x_dev, const float* w_hwio_dev, const float* bias_
   a.y = y_dev; a.B = B; a.H = H; a.W = W; a.Cin = Cin; a.Cout = Cout; a.size = size;
   a.stride = stride; a.padding = padding; a.relu = relu; a.y_cstride = y_cstride; a.y_coff = y_coff;
   return launch_conv_simt(a, (cudaStream_t)stream);
-}
-
-
-int sqdet_conv3x3_halo(const float* x_dev, const float* w_hwio_dev, const float* bias_dev,
-                       const float* scale_dev, const float* shift_dev, float* y_dev, int B, int H,
-                       int W, int Cin, int Cout, int relu, int y_cstride, int y_coff, void* stream_v) {
-  if (!x_dev || !w_hwio_dev || !y_dev)
-    return fail(SQDET_ERR_INVALID_ARG, "sqdet_conv3x3_halo: null pointer");
-  if (B <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0)
-    return fail(SQDET_ERR_INVALID_ARG, "sqdet_conv3x3_halo: non-positive dimension");
-  cudaStream_t stream = (cudaStream_t)stream_v;
-  HaloConvPlan plan;
-  int rc = halo_conv_plan(&plan, B, H, W, Cin, Cout, relu, scale_dev != nullptr, y_cstride, y_coff,
-                          x_dev, y_dev);
-  if (rc < 0) return rc;
-  if (rc == 0) return fail(SQDET_ERR_UNSUPPORTED, "sqdet_conv3x3_halo: shape not taken by the halo kernel");
-  std::vector<float> w((size_t)9 * Cin * Cout), b(Cout, 0.f), sc, sh;
-  cudaError_t ce = cudaMemcpy(w.data(), w_hwio_dev, w.size() * sizeof(float), cudaMemcpyDeviceToHost);
-  if (ce == cudaSuccess && bias_dev)
-    ce = cudaMemcpy(b.data(), bias_dev, Cout * sizeof(float), cudaMemcpyDeviceToHost);
-  if (ce == cudaSuccess && scale_dev) {
-    sc.resize(Cout); sh.resize(Cout);
-    ce = cudaMemcpy(sc.data(), scale_dev, Cout * sizeof(float), cudaMemcpyDeviceToHost);
-    if (ce == cudaSuccess) ce = cudaMemcpy(sh.data(), shift_dev, Cout * sizeof(float), cudaMemcpyDeviceToHost);
-  }
-  if (ce != cudaSuccess) {
-    halo_conv_release(&plan);
-    return cuda_fail(ce, "sqdet_conv3x3_halo: parameter download");
-  }
-  rc = halo_conv_pack_weights(&plan, w.data(), bias_dev ? b.data() : nullptr);
-  if (!rc && scale_dev) rc = halo_conv_set_affine(&plan, sc.data(), sh.data());
-  if (!rc) rc = launch_halo_conv(plan, stream);
-  ce = cudaStreamSynchronize(stream);
-  halo_conv_release(&plan);
-  if (rc) return rc;
-  if (ce != cudaSuccess) return cuda_fail(ce, "sqdet_conv3x3_halo sync");
-  return SQDET_OK;
 }
 
 /* SqueezeDet._fire_layer as ONE stage-isolated call (src/nets/squeezeDet.py:81-106). */

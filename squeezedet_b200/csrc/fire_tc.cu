@@ -87,9 +87,6 @@ struct FireParams {
   int sq_seg;              // squeeze stages (32 channels each) per accumulation segment: 3, or 4 with sq_on_split
   int sq_on_split;         // 1: the two splitter groups drain the squeeze accumulators (single-segment squeezes,
                            // S = 16): takes 40 % of the work off the drain warpgroups, which bounded fire2/3
-  int wg_perm;             // role of physical warpgroup i in bits [4i, 4i+4): 0,1 drains, 2 splitter A + TMA
-                           // producer, 3 splitter B + MMA issuer (issue arbitration favours high warp ids)
-  int sq_cat;              // squeeze MMAs as a_hi x [b_hi | b_lo] (N = 2S) + a_lo x b_hi: 2 per K step
   int ntiles_w;            // expand weight tiles in total
   int lo_rows_sq, lo_rows_e;   // rows between the hi and the lo copy in the packed matrices
   int tmem_cols;
@@ -175,9 +172,8 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
   uint64_t* tempty = sqfull + 10;                // [2]  expand drains -> MMA
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sqfull + 12);
 
-  pdl_trigger();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int role = (p.wg_perm >> (4 * (warp >> 2))) & 15;    // of this warpgroup, see FireParams
+  const int role = warp >> 2;   // 0,1 drains, 2 splitter A + TMA producer, 3 splitter B + MMA issuer
   const bool ctl = (warp & 3) == 3;                          // fourth warp of a splitter warpgroup
   const int S = p.S, Ne = p.Ne;
   const int kch = p.Cin >> 5;                    // 32-channel K chunks of the squeeze
@@ -207,12 +203,9 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();      // prologue overlapped the previous kernel's tail (PDL); global memory from here on
   // TMEM columns: [0, 2S) squeeze accumulators (M tile 0 | 1), [2S, 2S + 2Ne) expand accumulators
   // (two buffers), then one [a_hi | a_lo] = 64-column A slot per squeeze stage
-  // (with sq_cat the squeeze accumulators are 2S wide: [hi x hi + lo x hi | hi x lo])
-  const int SW = p.sq_cat ? 2 * S : S;
-  const uint32_t col_e = (uint32_t)(2 * SW), col_a = (uint32_t)(2 * SW + 2 * Ne);
+  const uint32_t col_e = (uint32_t)(2 * S), col_a = (uint32_t)(2 * S + 2 * Ne);
 
 #define FF_TILE_DECODE(item_)                          \
   int tile_ = (item_);                                 \
@@ -297,8 +290,6 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
       // ================================ MMA issuer (warp 15) ==================================
       const uint32_t idesc_s = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(S >> 3) << 17) |
                                ((uint32_t)(128 >> 4) << 24);
-      const uint32_t idesc_s2 = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)((2 * S) >> 3) << 17) |
-                                ((uint32_t)(128 >> 4) << 24);
       const uint32_t idesc_e = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(Ne >> 3) << 17) |
                                ((uint32_t)(128 >> 4) << 24);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
@@ -322,7 +313,7 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
             FF_WAIT(w_sqempty, &sqempty[mt], (use & 1u) ^ 1u);
             if (mt) ++sq_use1; else ++sq_use0;
             tc_fence_after();
-            const uint32_t d_tmem = tmem_u + (uint32_t)(mt * SW);
+            const uint32_t d_tmem = tmem_u + (uint32_t)(mt * S);
             for (int kc = seg0; kc < kch && kc < seg0 + p.sq_seg; ++kc) {
               FF_WAIT(w_split, &ssplit[rs.s], rs.ph);
               tc_fence_after();
@@ -335,15 +326,9 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
                 for (int j = 0; j < 4; ++j) {
                   const uint64_t dbh = dsw_hi | (uint64_t)(b_hi + 2 * j);
                   const uint64_t dbl = dsw_hi | (uint64_t)(b_lo + 2 * j);
-                  if (p.sq_cat) {
-                    // the hi and lo weight tiles are adjacent rows of the stage: one N = 2S operand
-                    umma_tf32_ts(d_tmem, a_hi + 8 * j, dbh, idesc_s2, (kc != seg0 || j != 0) ? 1u : 0u);
-                    umma_tf32_ts(d_tmem, a_lo + 8 * j, dbh, idesc_s, 1u);
-                  } else {
-                    umma_tf32_ts(d_tmem, a_lo + 8 * j, dbh, idesc_s, (kc != seg0 || j != 0) ? 1u : 0u);
-                    umma_tf32_ts(d_tmem, a_hi + 8 * j, dbl, idesc_s, 1u);
-                    umma_tf32_ts(d_tmem, a_hi + 8 * j, dbh, idesc_s, 1u);
-                  }
+                  umma_tf32_ts(d_tmem, a_lo + 8 * j, dbh, idesc_s, (kc != seg0 || j != 0) ? 1u : 0u);
+                  umma_tf32_ts(d_tmem, a_hi + 8 * j, dbl, idesc_s, 1u);
+                  umma_tf32_ts(d_tmem, a_hi + 8 * j, dbh, idesc_s, 1u);
                 }
                 umma_commit(&sempty[rs.s]);
               }
@@ -494,15 +479,13 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
         mbar_wait(&sqfull[sg], sqn & 1u);
         ++sqn;
         tc_fence_after();
-        uint32_t v[16], v2[16];
-        const uint32_t trow = tmem_base + lane_sel + (uint32_t)(sg * SW);
+        uint32_t v[16];
+        const uint32_t trow = tmem_base + lane_sel + (uint32_t)(sg * S);
         tmem_ld16_nowait(trow, v);
-        if (p.sq_cat) tmem_ld16_nowait(trow + 16u, v2);
         tmem_wait_ld();
         tc_fence_before();
         mbar_arrive(&sqempty[sg]);
-        const float gain = 1.f + p.bias_comp * (float)((p.sq_cat ? 8 : 12) * kch);
-        const float gain2 = 1.f + p.bias_comp * (float)(4 * kch);
+        const float gain = 1.f + p.bias_comp * (float)(12 * kch);
         const int gy = h0 - 1 + FF_MT_H * sg + hl, gx = w0 - 1 + wx;
         const bool inside = gy >= 0 && gy < p.H && gx >= 0 && gx < p.W;
         if (row_ok) {
@@ -514,8 +497,7 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
             float o[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
-              float a = __uint_as_float(v[c4 * 4 + e]) * gain;
-              if (p.sq_cat) a = fmaf(__uint_as_float(v2[c4 * 4 + e]), gain2, a);
+              const float a = __uint_as_float(v[c4 * 4 + e]) * gain;
               o[e] = inside ? fmaxf(a + bb[e], 0.f) : 0.f;
             }
             float4 hi, lo;
@@ -566,24 +548,18 @@ fire_fused_kernel(const __grid_constant__ FireParams p) {
         FF_WAIT(w_sqfull, &sqfull[g], sqn & 1u);
         tc_fence_after();
         const int nst = (kch - seg0) < p.sq_seg ? (kch - seg0) : p.sq_seg;
-        // chained MMAs per accumulator column in this segment: 3 per K step (sq_cat: 2 in the
-        // [hi x hi + lo x hi] half, 1 in the [hi x lo] half)
-        const float gain = 1.f + p.bias_comp * (float)((p.sq_cat ? 8 : 12) * nst);
-        const float gain2 = 1.f + p.bias_comp * (float)(4 * nst);
-        const uint32_t trow = tmem_base + lane_sel + (uint32_t)(g * SW);
+        // chained MMAs per accumulator column in this segment: 3 per K step
+        const float gain = 1.f + p.bias_comp * (float)(12 * nst);
+        const uint32_t trow = tmem_base + lane_sel + (uint32_t)(g * S);
 #pragma unroll
         for (int c0 = 0; c0 < FF_MAX_S; c0 += 16) {
           if (c0 < S) {                            // warp-uniform
-            uint32_t v[16], v2[16];
+            uint32_t v[16];
             tmem_ld16_nowait(trow + (uint32_t)c0, v);
-            if (p.sq_cat) tmem_ld16_nowait(trow + (uint32_t)(S + c0), v2);
             tmem_wait_ld();
 #pragma unroll
-            for (int e = 0; e < 16; ++e) {
-              float a = fmaf(__uint_as_float(v[e]), gain, seg0 == 0 ? 0.f : acc[c0 + e]);
-              if (p.sq_cat) a = fmaf(__uint_as_float(v2[e]), gain2, a);
-              acc[c0 + e] = a;
-            }
+            for (int e = 0; e < 16; ++e)
+              acc[c0 + e] = fmaf(__uint_as_float(v[e]), gain, seg0 == 0 ? 0.f : acc[c0 + e]);
           }
         }
         tc_fence_before();
@@ -740,18 +716,14 @@ static void release_fire(void** impl) {
   *impl = nullptr;
 }
 
-static int env_int(const char* name, int dflt) {
-  const char* a = getenv(name);
-  return a ? atoi(a) : dflt;
-}
-
 }  // namespace
 
 int fused_fire_plan(FusedFirePlan* plan, int B, int H, int W, int Cin, int S, int E1, int E3,
                     const float* x_dev, float* y_dev) {
   plan->enabled = false;
   plan->impl = nullptr;
-  if (!env_int("SQDET_FUSED_FIRE", 1)) return 0;
+  static const int env_fused = env_int("SQDET_FUSED_FIRE", 1);
+  if (!env_fused) return 0;
   // shapes this kernel takes (everything else stays on the squeeze + expand-pair launches)
   if (Cin % 32 != 0 || Cin < 32 || S % 16 != 0 || S < 16 || S > FF_MAX_S) return 0;
   if (E1 % 32 != 0 || E3 % 32 != 0 || E1 < 32 || E3 < 32 || E1 + E3 > 512) return 0;
@@ -784,28 +756,18 @@ int fused_fire_plan(FusedFirePlan* plan, int B, int H, int W, int Cin, int S, in
   P.q_half = (S / 4) * FF_QCH;
   P.q_bytes = 2 * P.q_half;
   P.sq_stage = FF_SQ_A + 2 * S * 128;
-  {
-    const char* a = getenv("SQDET_FF_PERM");
-    P.wg_perm = a ? (int)strtol(a, nullptr, 16) : 0x3210;
-  }
-  P.bias_comp = 1.4e-8f;
-  {
-    const char* a = getenv("SQDET_TC_BIAS_COMP");
-    if (a) P.bias_comp = (float)atof(a);
-  }
+  static const float env_comp = env_float("SQDET_TC_BIAS_COMP", 1.4e-8f);
+  P.bias_comp = env_comp;
   // shared-memory plan: the deepest configuration that fits 227 KB, in order of preference
   const int fixed = FF_PAR_FLOATS * 4 + 1024 /*barriers*/;
   const bool can_reside = (long long)tiles * P.ew_tile <= 120 * 1024;
-  // squeeze MMAs as 2 per K step (a_hi x [b_hi | b_lo] at N = 2S, a_lo x b_hi at N = S): opt-in, measured
-  // neutral to -3 % on fire2/3 (profiles/r2_fused_fire.txt) - the drains, not the MMA count, bound them
-  P.sq_cat = (S == 16 && env_int("SQDET_FF_SQCAT", 0)) ? 1 : 0;
-  const int SWh = P.sq_cat ? 2 * S : S;
   // squeeze drain on the splitter groups: single-segment squeezes with S = 16 (fire2/3: Cin <= 128 as
   // ONE segment of up to 4 stages = 48 chained MMAs).  OPT-IN: parity-green (tests/test_gpu_fire.py)
   // and -15 % / -6 % on fire2 / fire3 in the per-op timing (profiles/r2_fused_fire.txt), but the one
   // bench.py run made with it did not finish inside its time limit and the GPU budget of the round
   // ended before that could be explained - off until it is.
-  P.sq_on_split = (S == 16 && Cin <= 128 && env_int("SQDET_FF_SQSPLIT", 0)) ? 1 : 0;
+  static const int env_sqsplit = env_int("SQDET_FF_SQSPLIT", 0);
+  P.sq_on_split = (S == 16 && Cin <= 128 && env_sqsplit) ? 1 : 0;
   P.sq_seg = P.sq_on_split ? 4 : 3;
   struct Cand { int nq, nsq, nring, store_ring; };
   // deepest squeeze ring first (measured: with 2-3 stages the MMA warp waits on the TMA -> splitter
@@ -813,17 +775,11 @@ int fused_fire_plan(FusedFirePlan* plan, int B, int H, int W, int Cin, int S, in
   const Cand cands[] = {{2, 4, 4, 2}, {2, 4, 4, 1}, {2, 4, 3, 1}, {2, 3, 4, 1}, {2, 3, 3, 1}, {2, 3, 2, 1},
                         {1, 4, 4, 1}, {1, 3, 4, 1}, {1, 3, 3, 1}, {2, 2, 4, 1}, {2, 2, 3, 1}, {1, 2, 4, 1},
                         {1, 2, 3, 1}, {1, 2, 2, 1}};
-  const int force_nq = env_int("SQDET_FF_NQ", 0), force_res = env_int("SQDET_FF_RESIDENT", -1);
-  const int force_nsq = env_int("SQDET_FF_NSQ", 0), force_ring = env_int("SQDET_FF_NRING", 0);
   bool placed = false;
   for (int pass = 0; pass < 2 && !placed; ++pass) {
-    const bool resident = pass == 0 ? (can_reside && force_res != 0) : false;
+    const bool resident = pass == 0 && can_reside;   // weights resident first, else streamed
     if (pass == 0 && !resident) continue;
-    if (pass == 1 && force_res == 1) break;
     for (const Cand& c : cands) {
-      if (force_nq && c.nq != force_nq) continue;
-      if (force_nsq && c.nsq != force_nsq) continue;
-      if (force_ring && !resident && c.nring != force_ring) continue;
       // the exact shared-memory map of this candidate (same arithmetic as below)
       auto up1k = [](long long v) { return (v + 1023) & ~1023LL; };
       long long off = up1k((long long)c.nsq * P.sq_stage);
@@ -832,7 +788,7 @@ int fused_fire_plan(FusedFirePlan* plan, int B, int H, int W, int Cin, int S, in
       off = up1k(off + (long long)c.nq * P.q_bytes);
       off += fixed + 16 + 1024 /*base alignment*/;
       if (off > 232448) continue;
-      if (2 * SWh + 2 * Ne + 64 * c.nsq > 512) continue;
+      if (2 * S + 2 * Ne + 64 * c.nsq > 512) continue;
       P.nq = c.nq; P.nsq = c.nsq; P.nring = resident ? 1 : c.nring; P.store_ring = c.store_ring;
       P.resident = resident ? 1 : 0;
       placed = true;
@@ -855,7 +811,7 @@ int fused_fire_plan(FusedFirePlan* plan, int B, int H, int W, int Cin, int S, in
   }
   {
     int cols = 32;
-    while (cols < 2 * SWh + 2 * Ne + 64 * P.nsq) cols <<= 1;
+    while (cols < 2 * S + 2 * Ne + 64 * P.nsq) cols <<= 1;
     P.tmem_cols = cols;
   }
   int dev = 0, sms = 148;
@@ -948,8 +904,7 @@ int launch_fused_fire(const FusedFirePlan& plan, cudaStream_t stream) {
   const FireImpl* im = static_cast<const FireImpl*>(plan.impl);
   if (!im) return fail(SQDET_ERR_STATE, "no fused fire plan");
   FireParams prm = im->prm;
-  static int debug = -1;
-  if (debug < 0) debug = env_int("SQDET_TC_DEBUG", 0);
+  static const int debug = env_int("SQDET_TC_DEBUG", 0);
   long long* dbg = nullptr;
   const int nb = (int)im->grid.x;
   if (debug) {

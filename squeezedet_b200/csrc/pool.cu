@@ -23,8 +23,6 @@ __device__ __forceinline__ float4 ld_stream(const float4* p) {
 __global__ void __launch_bounds__(256)
 maxpool_vec4_kernel(const float* __restrict__ x, float* __restrict__ y, int B, int H, int W,
                     int C4, int k, int stride, int pad_t, int pad_l, int Ho, int Wo) {
-  pdl_trigger();
-  pdl_wait();
   const long long total = (long long)B * Ho * Wo * C4;
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
@@ -60,8 +58,6 @@ template <int K>
 __global__ void __launch_bounds__(256)
 maxpool_s2_vec4_kernel(const float* __restrict__ x, float* __restrict__ y, int B, int H, int W,
                        int C4, int pad_t, int pad_l, int Ho, int Wo) {
-  pdl_trigger();
-  pdl_wait();
   const int total = B * Ho * Wo * C4;
   const float4* __restrict__ x4 = reinterpret_cast<const float4*>(x);
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
@@ -102,8 +98,6 @@ maxpool_s2_vec4_kernel(const float* __restrict__ x, float* __restrict__ y, int B
 __global__ void __launch_bounds__(256)
 maxpool_scalar_kernel(const float* __restrict__ x, float* __restrict__ y, int B, int H, int W,
                       int C, int k, int stride, int pad_t, int pad_l, int Ho, int Wo) {
-  pdl_trigger();
-  pdl_wait();
   const long long total = (long long)B * Ho * Wo * C;
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
@@ -131,8 +125,6 @@ maxpool_scalar_kernel(const float* __restrict__ x, float* __restrict__ y, int B,
 __global__ void __launch_bounds__(256)
 add_relu_kernel(const float* __restrict__ a, const float* __restrict__ b,
                 float* __restrict__ y, long long n4, long long n) {
-  pdl_trigger();
-  pdl_wait();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n4) {
     const float4 p = ld_stream(reinterpret_cast<const float4*>(a) + i);
@@ -275,13 +267,8 @@ int launch_maxpool(const float* x, float* y, int B, int H, int W, int C, int siz
   long long blocks = (total + 255) / 256;
   const long long cap = 148LL * 8 * 16;   // grid-stride beyond 16 waves of 8 CTAs/SM
   if (blocks > cap) blocks = cap;
-  static int env_fast = -1;
-  if (env_fast < 0) {
-    const char* a = getenv("SQDET_POOL_FAST");
-    env_fast = a ? atoi(a) : 1;
-  }
   const long long in_elems = (long long)B * H * W * (C / 4);
-  if (vec && env_fast && stride == 2 && (size == 2 || size == 3) && total < (1LL << 30) &&
+  if (vec && stride == 2 && (size == 2 || size == 3) && total < (1LL << 30) &&
       in_elems < (1LL << 30)) {
     if (size == 3)
       SQ_CUDA(launch_kernel(maxpool_s2_vec4_kernel<3>, dim3((unsigned)blocks), dim3(256), 0, stream, x, y,

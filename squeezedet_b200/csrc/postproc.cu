@@ -32,8 +32,6 @@ interpret_kernel(const float* __restrict__ preds, const float* __restrict__ anch
                  float* __restrict__ boxes, float* __restrict__ probs,
                  long long* __restrict__ cls, int B, int A, int K, int C, float wm1,
                  float hm1, float exp_thresh, float slope) {
-  pdl_trigger();
-  pdl_wait();
   const long long total = (long long)B * A;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= total) return;
@@ -90,8 +88,6 @@ interpret_kernel(const float* __restrict__ preds, const float* __restrict__ anch
 __global__ void __launch_bounds__(256)
 rescale_boxes_kernel(float4* __restrict__ boxes, const float* __restrict__ scales, int A,
                      long long total) {
-  pdl_trigger();
-  pdl_wait();
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= total) return;
   const int b = (int)(idx / A);
@@ -149,8 +145,6 @@ filter_kernel(const float* __restrict__ boxes, const float* __restrict__ probs,
               const long long* __restrict__ cls, int A, int classes, int top_n,
               float prob_thresh, float nms_thresh, sqdet_det* __restrict__ dets,
               int* __restrict__ counts, int max_dets) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ unsigned long long s_key[FCAP];   // (order_key << 32) | (~anchor)
   __shared__ float4 s_box[FCAP];
   __shared__ int s_cls[FCAP];

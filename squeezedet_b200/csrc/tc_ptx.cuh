@@ -101,75 +101,6 @@ __device__ __forceinline__ void tma_store_wait_read_all() {
 __device__ __forceinline__ void tma_store_wait_all() {
   asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
-// 2-D TMA load multicast to every CTA of the cluster in `mask` (same smem offset and same
-// mbarrier offset in each destination CTA).
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar,
-                                               int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes"
-      ".multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(dst)),
-      "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 "
-      "[%0], %1;" ::"r"(smem_u32(bar)),
-      "h"(mask)
-      : "memory");
-}
-// ---- cta_group::2 (CTA-pair MMA): each CTA holds 128 rows of A in its own TMEM and HALF of
-// the B tile (N/2 rows) in its own smem; the leader CTA issues one M=256 MMA for the pair, so
-// the per-SM B smem traffic (reads and TMA fills) halves.
-__device__ __forceinline__ void tmem_alloc_2(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                   smem_u32(dst_smem)),
-               "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void umma_tf32_ts_2(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc,
-                                               uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], [%1], %2, %3, p;\n\t"
-      "}" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_2(uint64_t* bar) {   // arrives in BOTH CTAs of the pair
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 "
-      "[%0], %1;" ::"r"(smem_u32(bar)),
-      "h"((uint16_t)3)
-      : "memory");
-}
-// arrive on the mbarrier at the same smem offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t cta) {
-  asm volatile(
-      "{\n\t"
-      ".reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t"
-      "}" ::"r"(smem_u32(bar)),
-      "r"(cta)
-      : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
                    smem_u32(dst_smem)),

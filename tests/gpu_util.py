@@ -30,27 +30,6 @@ def conv2d_gpu(x, w, b=None, stride=1, padding='SAME', relu=True, scale=None, sh
   return dy.to_numpy(np.float32, (B, Ho, Wo, cs))
 
 
-def conv3x3_halo_gpu(x, w, b=None, relu=True, scale=None, shift=None, y_cstride=None, y_coff=0,
-                     device=0, y_init=None):
-  """sqdet_conv3x3_halo: the halo-tile tensor-core path of a 3x3 / stride 1 / SAME conv."""
-  lib = _lib.load()
-  B, H, W, Cin = x.shape
-  Cout = w.shape[3]
-  cs = y_cstride or Cout
-  dx = DeviceBuffer.from_numpy(x.astype(np.float32), device)
-  dw = DeviceBuffer.from_numpy(w.astype(np.float32), device)
-  db = DeviceBuffer.from_numpy(b.astype(np.float32), device) if b is not None else None
-  dsc = DeviceBuffer.from_numpy(scale.astype(np.float32), device) if scale is not None else None
-  dsh = DeviceBuffer.from_numpy(shift.astype(np.float32), device) if shift is not None else None
-  y0 = y_init if y_init is not None else np.full((B, H, W, cs), np.nan, np.float32)
-  dy = DeviceBuffer.from_numpy(y0, device)
-  _lib.check(lib.sqdet_conv3x3_halo(dx.ptr, dw.ptr, db.ptr if db else None, dsc.ptr if dsc else None,
-                                    dsh.ptr if dsh else None, dy.ptr, B, H, W, Cin, Cout, int(relu),
-                                    cs, y_coff, None))
-  _lib.check(lib.sqdet_stream_sync(device, None))
-  return dy.to_numpy(np.float32, (B, H, W, cs))
-
-
 def maxpool_gpu(x, k, stride, padding, device=0):
   lib = _lib.load()
   import oracle
